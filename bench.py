@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: seconds of output audio synthesised per second (RTF^-1).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision fp32|fp16|bf16]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--precision fp32|fp16|bf16] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference        # the reference algorithm's CPU path (oracle port) on the SAME step, rank 0 only
 
@@ -155,12 +155,14 @@ def cpu_oracle_rate(cfg, T: int, reps: int, warmup: int, threads: int, warmup_T:
             phone, lens, pitch, pitchf, sid = synthetic.make_inputs(cfg, 1, Ti)
             noise = synthetic.draw_noise(cfg, 1, Ti, seed=7 + max(i - warmup, 0))     # first timed step = the g2 fixture's draw
             t0 = time.perf_counter()
-            o = rvc_oracle.infer(w, cfg, phone, lens, pitch, pitchf, sid, *noise)[0]
+            outs = rvc_oracle.infer(w, cfg, phone, lens, pitch, pitchf, sid, *noise)
             dt = time.perf_counter() - t0
             if i >= warmup:
                 times.append(dt)
             if i == warmup and check is not None:
-                check["first_timed_output"] = o[0, 0].numpy()
+                check["first_timed_output"] = outs[0][0, 0].numpy()
+            if check is not None:
+                check["last_timed"] = outs
     finally:
         torch.set_num_threads(prev)
     audio_s = T * cfg.upp / cfg.sr
@@ -299,6 +301,25 @@ def measured_traffic(precision: str):
 _REAL_STDOUT = None
 
 
+DUMP_BUDGET_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, outs):
+    """Writes what one `infer()` returned -- `(o, x_mask, (z, z_p, m_p, logs_p))` -- as `out_dir/<name>.npy` in float32, so
+    two builds run with the same arguments can be compared array for array.  Above 64 MB in all, every array keeps the same
+    fixed, seeded sample of its flattened elements."""
+    o, x_mask, (z, z_p, m_p, logs_p) = outs
+    arrays = {"audio": o, "x_mask": x_mask, "z": z, "z_p": z_p, "m_p": m_p, "logs_p": logs_p}
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    keep = min(1.0, DUMP_BUDGET_BYTES / sum(a.size * 4 for a in arrays.values()))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if keep < 1.0:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def claim_stdout():
     """stdout carries exactly ONE JSON line: everything libraries print there (NCCL's version banner under
     NCCL_DEBUG=VERSION, warnings of child tools) is sent to stderr for the lifetime of the process."""
@@ -335,7 +356,12 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-front-end", action="store_true")
     ap.add_argument("--no-extra-precision", action="store_true", help="skip the fp16 leg beside the bf16 headline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step's infer() returned as DIR/<name>.npy (float32, at most 64 MB in all; "
+                         "under torchrun, rank 0's outputs only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     cfg = NAMED_CONFIGS[args.config]
     T = int(round(args.seconds * 100))
@@ -355,11 +381,13 @@ def main():
         if rank != 0:
             return
         threads = os.cpu_count() or 1
-        steps, warm = max(1, args.steps), max(0, args.warmup)
+        steps, warm = args.steps, max(0, args.warmup)
         # every step is the product arm's step: one full infer() of T frames on all host cores (oracle port, fp32).
         # EXACTLY `steps` timed steps after `warm` untimed ones; value = audio produced / total time of the K steps
         chk = {}
         _, sample_s, times = cpu_oracle_rate(cfg, cpu_T, steps, warm, threads, check=chk)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, chk["last_timed"])
         rate = steps * sample_s / float(np.sum(times))
         sample = (f"oracle/rvc_oracle.py (fp32 PyTorch CPU restatement of the reference infer), {cpu_T} frames = {sample_s:.1f} s "
                   f"audio per step" + (" = the full step" if cpu_T == T else " (bounded sample of the step)"))
@@ -404,10 +432,12 @@ def main():
     lib = _lib.load()
 
     def step_resident():
-        return net.infer(*devin)[0]          # draws its noise with torch on the device, like the reference
+        return net.infer(*devin)             # draws its noise with torch on the device, like the reference
 
+    # the warm-up holds each step's outputs until the next step returns, as the timed loop does, so the allocator
+    # already has blocks for both when the timed region starts
     for _ in range(max(3, args.warmup)):
-        step_resident()
+        outs = step_resident()
     torch.cuda.synchronize()
 
     def barrier():
@@ -424,10 +454,13 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_resident()
+        outs = step_resident()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs)
+    del outs
     launches = net.last_launches * args.steps
     graph_replay = bool(getattr(net, "last_graph_replay", False))   # the timed steps ran as replays of the captured step
     # per-class kernel times: a second pass of the same K steps with a CUDA-event pair around every launch (the event

@@ -1,11 +1,14 @@
 """CPU: bench.py's contract pieces that need no GPU -- the reference arm prints exactly one JSON line with the agreed
-keys, and the algorithmic FLOP / byte models reproduce the figures of SURVEY.md §8(d) / DESIGN.md §4."""
+keys, `--dump-outputs` writes the same arrays on every run, and the algorithmic FLOP / byte models reproduce the figures of
+SURVEY.md §8(d) / DESIGN.md §4."""
 import json
 import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -31,6 +34,44 @@ def test_reference_arm_prints_one_json_line():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
                          capture_output=True, text=True, env=env, timeout=600, cwd=ROOT)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_reference_arm_dumps_its_last_timed_step(tmp_path):
+    """Two runs write the same arrays, and they are the oracle's outputs for the LAST timed step (the second of two: noise
+    seed 8), each under its own name."""
+    from oracle import rvc_oracle
+    from comfy_rvc_b200 import synthetic
+    args = [sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "0",
+            "--cpu-frames", "20", "--dump-outputs"]
+    env = dict(os.environ, RANK="0", WORLD_SIZE="1")
+    for d in ("a", "b"):
+        out = subprocess.run(args + [str(tmp_path / d)], capture_output=True, text=True, env=env, timeout=600, cwd=ROOT)
+        assert out.returncode == 0, out.stderr[-2000:]
+    cfg = NAMED_CONFIGS["48k_v2"]
+    w = rvc_oracle.fold_weight_norm(synthetic.make_state_dict(cfg))
+    inputs = synthetic.make_inputs(cfg, 1, 20)
+    step = lambda seed: rvc_oracle.infer(w, cfg, *inputs, *synthetic.draw_noise(cfg, 1, 20, seed=seed))
+    o, x_mask, (z, z_p, m_p, logs_p) = step(8)
+    want = {"audio": o, "x_mask": x_mask, "z": z, "z_p": z_p, "m_p": m_p, "logs_p": logs_p}
+    for name, ref in want.items():
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float32 and a.shape == tuple(ref.shape) and np.array_equal(a, b), name
+        np.testing.assert_allclose(a, ref.numpy(), rtol=1e-5, atol=1e-5, err_msg=name)
+    first = step(7)[0].numpy()                       # the first timed step's waveform is a different one
+    assert np.abs(np.load(tmp_path / "a" / "audio.npy") - first).max() > 1e-3
+    out = subprocess.run(args[:4] + ["--steps", "0"], capture_output=True, text=True, env=env, timeout=600, cwd=ROOT)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+
+
+def test_dump_outputs_samples_above_the_budget(tmp_path, monkeypatch):
+    monkeypatch.setattr(bench, "DUMP_BUDGET_BYTES", 4 * 1000)
+    outs = (torch.arange(3000.0).reshape(1, 1, 3000), torch.ones(1, 1, 10), tuple(torch.zeros(1, 4, 10) for _ in range(4)))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), outs)
+    a = np.load(tmp_path / "a" / "audio.npy")
+    total = sum(np.load(tmp_path / "a" / f"{n}.npy").nbytes for n in ("audio", "x_mask", "z", "z_p", "m_p", "logs_p"))
+    assert total <= 4 * 1000 and a.dtype == np.float32 and a.size > 900
+    assert np.all(np.diff(a) > 0) and np.array_equal(a, np.load(tmp_path / "b" / "audio.npy"))
 
 
 def test_algorithmic_flop_model_matches_survey():
