@@ -158,8 +158,9 @@ __device__ __forceinline__ void epilogue_generic16(const TcConvDesc& p, uint32_t
       }
   }
   if (p.div != 1.f) {
+    const float rd = 1.f / p.div;
 #pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = v[i] / p.div;
+    for (int i = 0; i < 16; ++i) v[i] = div_exact(v[i], p.div, rd);
   }
   if (p.mask_post && !valid) {
 #pragma unroll
@@ -1125,7 +1126,7 @@ cudaError_t launch_conv_tc(const TcConvDesc& d_in, int B, cudaStream_t st) {
       d.Lj <= 0 || d.L_in <= 0 || (d.a_mode != 1 && slab_rows_halo(d) > 127) || tap_halo(d) < 0 || d.tap_w < 0 ||
       d.a_mode < 0 || d.a_mode > 2 || (d.a_mode == 2 && d.tap_w <= 0) || d.a_nt_stride < 0 || (d.a_nt_stride > 0 && (!d.generic || d.G != 1)) ||
       (d.tap_w > 0 && (d.ntaps % d.tap_w != 0 || d.dil2 < (d.tap_w - 1) * d.dil)) || d.pad_period < 0 || (d.pad_period > 0 && !d.generic) || (d.accum && !d.y32) || B <= 0 || !d.x16 || !d.w16 ||
-      d.a_fp16 || (d.res16 && d.res32) || (d.acc_f16 && (d.generic || d.Cout_total % 8)))
+      d.a_fp16 || (d.res16 && d.res32) || (d.acc_f16 && (d.generic || d.Cout_total % 8)) || !tc_div_exact(d.div))
     return cudaErrorInvalidValue;
   EncodeTiledFn enc = encode_tiled();
   if (!enc) return cudaErrorNotSupported;

@@ -10,6 +10,8 @@ typedef rvcb200_tc_conv_desc TcConvDesc;
 
 constexpr int kPadF = 32;                                   // zero rows in front of every PV plane
 inline int pv_pitch_rows(long long L) { return (int)(((L + 127) / 128) * 128 + 128); }   // Lp
+// epilogue divisors (the branch mean 1 / n_res_kernels) that tc::div_exact reproduces bit for bit
+inline bool tc_div_exact(float d) { return d == 1.f || d == 2.f || d == 3.f || d == 4.f; }
 
 cudaError_t launch_conv_tc(const TcConvDesc& d, int B, cudaStream_t st);
 // debug: device buffer of 16 x grid uint64 that receives phase timestamps of the following launches (nullptr: off)

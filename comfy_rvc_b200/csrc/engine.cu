@@ -1046,10 +1046,13 @@ static int infer_impl(rvcb200_ctx* ctx, int32_t B, int32_t T, const float* phone
             if (final_branch && !last_stage) { o.y16 = N16; o.out_slope = 0.1f; }
             if (final_branch && last_stage && post_tc) {
               // the decoder's last tensor is consumed once, by conv_post, as lrelu_{0.01}(x) (models.py:561): it leaves as
-              // that 16-bit channels-last operand; the planar branch sum is not written back unless a test taps it
+              // that 16-bit channels-last operand
               o.y16 = N16; o.out_slope = 0.01f;
-              o.acc_nostore = (o.accum && tp.find(S("dec.stage.%d", i).c_str()) == nullptr) ? 1 : 0;
             }
+            // the stage's result leaves as the 16-bit stream N16 (the next ups / conv_post reads it) and the next stage's
+            // first branch overwrites ACC32: the planar branch sum is not written back unless a test taps it
+            if (final_branch && o.y16)
+              o.acc_nostore = (o.accum && tp.find(S("dec.stage.%d", i).c_str()) == nullptr) ? 1 : 0;
           } else {
             o.y16 = ynew; o.out_slope = 0.1f;
           }

@@ -9,7 +9,8 @@
 //   * one "tile" is MSUB x 128 time rows: one activation slab (MSUB*128 + halo rows per 64-channel k-block, loaded
 //     by <= 3 TMA boxes) feeds MSUB accumulators, so barrier round trips, ring updates and -- when the weights do
 //     not fit in shared memory (C = 128, k = 7/11; C = 256) -- the weight stream are amortised over MSUB x more work,
-//   * the epilogue software-pipelines the fp32 residual loads one 32-column chunk ahead of the TMEM reads,
+//   * the epilogue moves its 16-bit residual and output as TMA boxes (the residual one 32-column chunk ahead of the
+//     TMEM reads), at every C,
 //   * the bias lives in shared memory.
 // Layouts, epilogue semantics and the weight packing are those of conv_tc.cu (see its header).
 #include "tc_ptx.cuh"
@@ -39,9 +40,9 @@ constexpr RbPlan rb_plan(int C, int NTAPS, int DIL, int MSUB) {
   q.a_bytes = q.nbox * q.rb * 128;
   q.w_bytes = C * 128;
   q.nw = q.nkb * NTAPS;
-  // epilogue staging (C <= 128): per warp 2 residual boxes + out_slots output boxes
-  q.out_slots = C == 128 ? 1 : 2;
-  q.epi_bytes = C <= 128 ? 8 * (2 + q.out_slots) * kEpiBox : 0;
+  // epilogue staging: per warp 2 residual boxes + out_slots output boxes
+  q.out_slots = C >= 128 ? 1 : 2;
+  q.epi_bytes = 8 * (2 + q.out_slots) * kEpiBox;
   q.budget = 218 * 1024 - q.epi_bytes;
   q.stat = (q.nw * q.w_bytes <= 96 * 1024 && (q.budget - q.nw * q.w_bytes) / q.a_bytes >= 2) ? 1 : 0;
   q.nb = q.stat ? q.nw : (C >= 256 ? 3 : (C == 128 ? 4 : 6));
@@ -74,7 +75,6 @@ struct RbCfg {
   static constexpr bool STAT = P.stat != 0;                // weights resident for the whole CTA
   static constexpr int NB = P.nb;
   static constexpr int NA = P.na_fit > 6 ? 6 : P.na_fit;
-  static constexpr bool EPI_TMA = C <= 128;                // 16-bit epilogue I/O staged in smem and moved by TMA
   static constexpr int OUT_SLOTS = P.out_slots;
   static constexpr int EPI_WARP_BYTES = (2 + OUT_SLOTS) * kEpiBox;
   static constexpr int EPI_BYTES = P.epi_bytes;
@@ -251,9 +251,9 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
     }
   } else {
     // ============== epilogue: two groups of 4 warps, group e drains accumulator buffer e ==================
-    // 16-bit I/O (C <= 128): thread = TMEM lane = time row, so direct global accesses would be 16-byte pieces 2*C bytes
-    // apart -- 32 L2 requests per warp instruction; measured ~0.37 requests/clk/SM whatever the byte count, the limit
-    // of every epilogue-heavy shape (profiles/r1_conv_shapes_v8_*.jsonl).  Instead each warp moves [32 rows][32 channels]
+    // 16-bit I/O: thread = TMEM lane = time row, so direct global accesses would be 16-byte pieces 2*C bytes apart --
+    // 32 L2 requests per warp instruction; measured ~0.37 requests/clk/SM whatever the byte count, the limit of every
+    // epilogue-heavy shape (profiles/r1_conv_shapes_v8_*.jsonl).  Instead each warp moves [32 rows][32 channels]
     // boxes with TMA: the residual box lands in a SWIZZLE_64B staging slot (2 slots, loaded one chunk ahead), the
     // 16-bit output box is written to a staging slot by the lanes (conflict-free under the swizzle) and stored by one
     // lane.  The fp16 planar branch sum keeps the direct path: its warp accesses are 512 B contiguous.
@@ -266,7 +266,7 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
     const size_t pitch_o = (size_t)p.Lp_out * 16;   // bytes per planar-vector plane
     const bool obf = p.out_bf16 != 0;
     const float slope = p.out_slope;
-    const float inv_div = p.div;                    // divide (not multiply by reciprocal): matches the fp32 path
+    const float div = p.div, rdiv = 1.f / p.div;    // branch mean: exact quotient without a divide (div_exact)
     const float neg_scale = p.res_neg_scale == 0.f ? 1.f : p.res_neg_scale;
     const bool has_r16 = p.res16 != nullptr;
     const bool has_y16 = p.y16 != nullptr;
@@ -289,24 +289,13 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
       const int row_base = wrow0 + lane;
       const uint32_t tbase = tmem_base + ((uint32_t)(qd * 32) << 16) + (uint32_t)(eg * MSUB * C);
       unsigned char* acc = has_acc ? reinterpret_cast<unsigned char*>(p.y32) + (size_t)b * (C / 8) * pitch_o : nullptr;
-      unsigned char* y16 = has_y16 ? reinterpret_cast<unsigned char*>(p.y16) + (size_t)b * (size_t)p.Lj * C * 2 : nullptr;
-      const unsigned char* r16 = has_r16 ? reinterpret_cast<const unsigned char*>(p.res16) + (size_t)b * (size_t)p.Lj * C * 2 : nullptr;
 
-      uint4 rq[16];   // [0,8): direct residual, 2 slots x 4 words (C = 256); [8,16): branch-sum prefetch, 2 slots x 4 words
+      uint4 rq[8];    // branch-sum prefetch, 2 slots x 4 words
       auto issue_box = [&](int ci, int slot) {       // one lane: residual box of chunk ci -> staging slot
         const int ms = ci / CPS, c0 = (ci - ms * CPS) * 32;
         uint64_t* bar = &my_res_full[slot];
         mbar_expect_tx(bar, kEpiBox);
         tma_load_3d(my_stage + slot * kEpiBox, &tmR, c0, wrow0 + ms * 128, (int)b, bar);
-      };
-      auto load_res = [&](int ci, int slot) {        // direct path (C = 256): this lane's 64 bytes of the residual row
-        const int ms = ci / CPS, c0 = (ci - ms * CPS) * 32;
-        const int row = row_base + ms * 128;
-        if (row < p.Lj) {
-          const uint4* q = reinterpret_cast<const uint4*>(r16 + ((size_t)row * C + c0) * 2);
-#pragma unroll
-          for (int k = 0; k < 4; ++k) rq[slot * 4 + k] = ld_nc_u4(q + k);
-        }
       };
       auto load_acc = [&](int ci, int slot) {
         const int ms = ci / CPS, c0 = (ci - ms * CPS) * 32;
@@ -314,17 +303,11 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
         if (row < p.Lj) {
           const unsigned char* q = acc + (size_t)(c0 / 8) * pitch_o + (size_t)(row + p.padf) * 16;
 #pragma unroll
-          for (int k = 0; k < 4; ++k) rq[8 + slot * 4 + k] = *reinterpret_cast<const uint4*>(q + (size_t)k * pitch_o);
+          for (int k = 0; k < 4; ++k) rq[slot * 4 + k] = *reinterpret_cast<const uint4*>(q + (size_t)k * pitch_o);
         }
       };
       // the first residual / branch-sum words are in flight before the MMAs of this tile finish
-      if (has_r16) {
-        if (K::EPI_TMA) {
-          if (lane == 0) { issue_box(0, 0); issue_box(1, 1); }
-        } else {
-          load_res(0, 0);
-        }
-      }
+      if (has_r16 && lane == 0) { issue_box(0, 0); issue_box(1, 1); }
       if (do_acc) load_acc(0, 0);
       mbar_wait(&acc_full[eg], (it >> 1) & 1u);
       tc_fence_after();
@@ -336,7 +319,6 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
           const int ms = ci / CPS, c0 = (ci - ms * CPS) * 32;
           const int row = row_base + ms * 128;
           const bool row_ok = row < p.Lj;
-          if (!K::EPI_TMA && has_r16 && ci + 1 < K::NCH) load_res(ci + 1, u ^ 1);
           if (do_acc && ci + 1 < K::NCH) load_acc(ci + 1, u ^ 1);
           uint32_t r[32];
           const uint32_t taddr = tbase + (uint32_t)(ms * C + c0);
@@ -392,28 +374,23 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
             }
           }
           if (has_r16) {
-            if (K::EPI_TMA) {
-              // residual box of this chunk: wait, read this lane's row, hand the slot back, refill it two chunks ahead
-              const unsigned char* box = my_stage + u * kEpiBox + sw_row;
-              mbar_wait(&my_res_full[u], rpar);
+            // residual box of this chunk: wait, read this lane's row, hand the slot back, refill it two chunks ahead
+            const unsigned char* box = my_stage + u * kEpiBox + sw_row;
+            mbar_wait(&my_res_full[u], rpar);
 #pragma unroll
-              for (int k = 0; k < 4; ++k)
-                add_res8(v + k * 8, *reinterpret_cast<const uint4*>(box + ((((uint32_t)k) ^ sw_x) << 4)), neg_scale);
-              __syncwarp();
-              if (lane == 0 && ci + 2 < K::NCH) issue_box(ci + 2, u);
-            } else {
-#pragma unroll
-              for (int k = 0; k < 4; ++k) add_res8(v + k * 8, rq[u * 4 + k], neg_scale);
-            }
+            for (int k = 0; k < 4; ++k)
+              add_res8(v + k * 8, *reinterpret_cast<const uint4*>(box + ((((uint32_t)k) ^ sw_x) << 4)), neg_scale);
+            __syncwarp();
+            if (lane == 0 && ci + 2 < K::NCH) issue_box(ci + 2, u);
           }
           if (has_acc) {
             if (do_acc) {
 #pragma unroll
-              for (int k = 0; k < 4; ++k) add_res8(v + k * 8, rq[8 + u * 4 + k], 1.f);
+              for (int k = 0; k < 4; ++k) add_res8(v + k * 8, rq[u * 4 + k], 1.f);
             }
-            if (inv_div != 1.f) {
+            if (div != 1.f) {
 #pragma unroll
-              for (int i = 0; i < 32; ++i) v[i] = v[i] / inv_div;
+              for (int i = 0; i < 32; ++i) v[i] = div_exact(v[i], div, rdiv);
             }
             if (row_ok && st_acc) {
               unsigned char* q = acc + (size_t)(c0 / 8) * pitch_o + (size_t)(row + p.padf) * 16;
@@ -425,9 +402,9 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
                 *reinterpret_cast<uint4*>(q + (size_t)k * pitch_o) = o;
               }
             }
-          } else if (inv_div != 1.f) {
+          } else if (div != 1.f) {
 #pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = v[i] / inv_div;
+            for (int i = 0; i < 32; ++i) v[i] = div_exact(v[i], div, rdiv);
           }
           if (has_y16) {
             uint4 o[4];
@@ -438,34 +415,28 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
               o[k8].z = pack2(obf, lrelu_max(v[k8 * 8 + 4], slope), lrelu_max(v[k8 * 8 + 5], slope));
               o[k8].w = pack2(obf, lrelu_max(v[k8 * 8 + 6], slope), lrelu_max(v[k8 * 8 + 7], slope));
             }
-            if (K::EPI_TMA) {
-              // stage the [32 rows][32 channels] box, then one lane stores it (rows >= L are clipped by the tensor map)
-              unsigned char* box = my_stage + (2 + (ocnt % K::OUT_SLOTS)) * kEpiBox;
-              if (lane == 0) bulk_wait_read<K::OUT_SLOTS - 1>();      // the store that last used this slot has read it
-              __syncwarp();
+            // stage the [32 rows][32 channels] box, then one lane stores it (rows >= L are clipped by the tensor map)
+            unsigned char* box = my_stage + (2 + (ocnt % K::OUT_SLOTS)) * kEpiBox;
+            if (lane == 0) bulk_wait_read<K::OUT_SLOTS - 1>();      // the store that last used this slot has read it
+            __syncwarp();
 #pragma unroll
-              for (int k = 0; k < 4; ++k) *reinterpret_cast<uint4*>(box + sw_row + ((((uint32_t)k) ^ sw_x) << 4)) = o[k];
-              fence_proxy_async();
-              __syncwarp();
-              if (lane == 0) {
-                tma_store_3d(&tmY, box, c0, wrow0 + ms * 128, (int)b);
-                bulk_commit();
-              }
-              ++ocnt;
-            } else if (row_ok) {
-              unsigned char* yr = y16 + ((size_t)row * C + c0) * 2;
-#pragma unroll
-              for (int k8 = 0; k8 < 4; ++k8) *reinterpret_cast<uint4*>(yr + k8 * 16) = o[k8];
+            for (int k = 0; k < 4; ++k) *reinterpret_cast<uint4*>(box + sw_row + ((((uint32_t)k) ^ sw_x) << 4)) = o[k];
+            fence_proxy_async();
+            __syncwarp();
+            if (lane == 0) {
+              tma_store_3d(&tmY, box, c0, wrow0 + ms * 128, (int)b);
+              bulk_commit();
             }
+            ++ocnt;
           }
         }
-        if (K::EPI_TMA && has_r16) rpar ^= 1u;
+        if (has_r16) rpar ^= 1u;
       }
       tc_fence_before();
       __syncwarp();
       if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&acc_empty[eg])) : "memory");
     }
-    if (K::EPI_TMA && lane == 0) bulk_wait_all();     // staged stores complete before the CTA's smem goes away
+    if (lane == 0) bulk_wait_all();     // staged stores complete before the CTA's smem goes away
   }
   // ------------------------------------ teardown -------------------------------------------------
   tc_fence_before();
@@ -514,21 +485,19 @@ cudaError_t launch_one(const TcConvDesc& d, int B, cudaStream_t st) {
     // epilogue boxes: [32 rows][32 channels] of the 16-bit channels-last residual / output, SWIZZLE_64B staging
     tmR = tmA;
     tmY = tmA;
-    if (K::EPI_TMA) {
-      cuuint64_t odims[3] = {(cuuint64_t)C, (cuuint64_t)d.Lj, (cuuint64_t)B};
-      cuuint64_t ostrides[2] = {(cuuint64_t)C * 2, (cuuint64_t)C * 2 * (cuuint64_t)d.Lj};
-      cuuint32_t obox[3] = {32, 32, 1};
-      if (d.res16 &&
-          enc(&tmR, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d.res16), odims, ostrides, obox, es,
-              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return cudaErrorInvalidValue;
-      if (d.y16 &&
-          enc(&tmY, d.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, d.y16, odims, ostrides,
-              obox, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return cudaErrorInvalidValue;
-    }
+    cuuint64_t odims[3] = {(cuuint64_t)C, (cuuint64_t)d.Lj, (cuuint64_t)B};
+    cuuint64_t ostrides[2] = {(cuuint64_t)C * 2, (cuuint64_t)C * 2 * (cuuint64_t)d.Lj};
+    cuuint32_t obox[3] = {32, 32, 1};
+    if (d.res16 &&
+        enc(&tmR, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d.res16), odims, ostrides, obox, es,
+            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+      return cudaErrorInvalidValue;
+    if (d.y16 &&
+        enc(&tmY, d.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, d.y16, odims, ostrides,
+            obox, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+      return cudaErrorInvalidValue;
   }
   static SmemOptIn opt;
   if (cudaError_t e = opt_in_smem(rbconv_tc_kernel<C, NTAPS, DIL, MSUB>, K::SMEM, opt)) return e;
@@ -570,6 +539,7 @@ bool rbconv_tc_supported(const TcConvDesc& d) {
   if (d.res32 || (d.y32 && !d.acc_f16)) return false;      // fp32 planar residual / output: generic kernel only
   if (d.tanh_out && (d.y16 || d.y32 || d.res16 || d.Cin > 128)) return false;       // conv_post mode: the only output
   if (d.acc_nostore && !(d.y32 && d.accum && d.y16)) return false;
+  if (!tc_div_exact(d.div)) return false;
   if (d.inj_har && (!d.inj_w || !d.inj_b || d.inj_k < 1 || d.inj_k > 4 || !(d.inj_cn == 32 || d.inj_cn == 64) ||
                     d.Cin % d.inj_cn != 0 || !d.y16 || d.y32 || d.res16 || d.tanh_out || d.inj_s < 1))
     return false;

@@ -395,7 +395,7 @@ rbpair_tc_kernel(const PairParams p, const __grid_constant__ CUtensorMap tmA, co
     const size_t pitch_o = (size_t)p.Lp_out * 16;   // bytes per planar-vector plane
     const bool obf = p.out_bf16 != 0;
     const float slope = p.out_slope;
-    const float inv_div = p.div;                    // divide (not multiply by reciprocal): matches the fp32 path
+    const float div = p.div, rdiv = 1.f / p.div;    // branch mean: exact quotient without a divide (div_exact)
     const float neg_scale = p.res_neg_scale == 0.f ? 1.f : p.res_neg_scale;
     const bool has_y16 = p.y16 != nullptr;
     const bool has_acc = p.y32 != nullptr;
@@ -475,9 +475,9 @@ rbpair_tc_kernel(const PairParams p, const __grid_constant__ CUtensorMap tmA, co
 #pragma unroll
             for (int k = 0; k < 4; ++k) add_res8(v + k * 8, aq[ci][k], 1.f);
           }
-          if (inv_div != 1.f) {
+          if (div != 1.f) {
 #pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = v[i] / inv_div;
+            for (int i = 0; i < 32; ++i) v[i] = div_exact(v[i], div, rdiv);
           }
           if (row_ok && st_acc) {
             unsigned char* q = acc + (size_t)(c0 / 8) * pitch_o + (size_t)(row + p.padf) * 16;
@@ -489,9 +489,9 @@ rbpair_tc_kernel(const PairParams p, const __grid_constant__ CUtensorMap tmA, co
               *reinterpret_cast<uint4*>(q + (size_t)k * pitch_o) = o;
             }
           }
-        } else if (inv_div != 1.f) {
+        } else if (div != 1.f) {
 #pragma unroll
-          for (int i = 0; i < 32; ++i) v[i] = v[i] / inv_div;
+          for (int i = 0; i < 32; ++i) v[i] = div_exact(v[i], div, rdiv);
         }
         if (has_y16) {
           // this lane's row of the [32 rows][32 channels] staging box of chunk ci (conflict-free under the swizzle)

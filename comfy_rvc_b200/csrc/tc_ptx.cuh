@@ -138,6 +138,17 @@ __device__ __forceinline__ void add_res8(float* v, const uint4& w, float neg_sca
   for (int i = 0; i < 8; ++i) v[i] += fminf(r[i], r[i] * neg_scale);
 }
 
+// v / d rounded to nearest, bit for bit as the IEEE divide, for d in {2, 3, 4} (tc_div_exact) and r = 1.f / d:
+// the remainder e = v - q0 * d is exact under the FMA, so one correction step gives the rounded quotient (checked over all
+// 2^32 inputs per divisor by tests/test_exact_div.py).  q0 is kept where e is zero -- the sign of -0 (fmaf(+0, r, -0) is
+// +0) -- or NaN -- v = +-inf (inf - inf) and v = NaN.  A plain divide is a div.rn.f32: an FCHK slow-path test plus a
+// branch per value.
+__device__ __forceinline__ float div_exact(float v, float d, float r) {
+  const float q0 = __fmul_rn(v, r);
+  const float e = __fmaf_rn(-q0, d, v);
+  return fabsf(e) > 0.f ? __fmaf_rn(e, r, q0) : q0;
+}
+
 // ---- bulk-tensor (TMA) stores from shared memory ----
 __device__ __forceinline__ void tma_store_3d(const CUtensorMap* tm, const void* src, int c0, int c1, int c2) {
   asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
@@ -247,8 +258,9 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvDesc& p, uint32_t tad
     }
   }
   if (p.div != 1.f) {
+    const float rd = 1.f / p.div;
 #pragma unroll
-    for (int i = 0; i < CH; ++i) v[i] = v[i] / p.div;
+    for (int i = 0; i < CH; ++i) v[i] = div_exact(v[i], p.div, rd);
   }
   if (y32 && p.acc_f16) {
 #pragma unroll
