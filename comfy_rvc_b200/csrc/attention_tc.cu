@@ -28,11 +28,7 @@
 // logits at that scale, Pband Ev is accumulated into O_0, O_1 is added in registers).  Three MMA-issuing warps: warp 1 /
 // warp 10 issue Q K^T for group 0 / 1, warp 11 issues P V and Pband Ev -- with ONE issuer the kernel was bound by that
 // thread's instruction stream (~145 SASS instructions, ~1200 cycles per key tile).
-#include <cuda.h>
-#include <cuda_fp16.h>
-
-#include "common.cuh"
-#include "conv_tc.cuh"
+#include "tc_ptx.cuh"
 
 namespace rvc {
 namespace {
@@ -46,94 +42,13 @@ constexpr uint32_t TM_O = 0, TM_R = 96, TM_Q = 192, TM_S = 256, TM_COLS = 512;
 constexpr float kTau = 4.f;                  // a row's running max is raised (and O rescaled) only when exceeded by more than this
 constexpr float kLog2e = 1.4426950408889634f;
 
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void bar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void bar_expect(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void bar_wait(uint64_t* bar, uint32_t parity) {
-  const uint32_t addr = s_u32(bar);
-  uint32_t done;
-  do {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t"
-        "}" : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-  } while (!done);
-}
-__device__ __forceinline__ void tma3(void* dst, const CUtensorMap* tm, int c0, int c1, int c2, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(s_u32(dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(s_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void tma2(void* dst, const CUtensorMap* tm, int c0, int c1, uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(s_u32(dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(s_u32(bar)), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ bool elect1() {
-  uint32_t pred;
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "elect.sync _|p, 0xffffffff;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t"
-      "}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint32_t a_lo, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      ".reg .b64 da, db;\n\t"
-      "mov.b64 da, {%1, %3};\n\t"
-      "mov.b64 db, {%2, %3};\n\t"
-      "setp.ne.b32 p, %5, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %4, p;\n\t"
-      "}" ::"r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(acc) : "memory");
-}
-// A operand in tensor memory (lane = row, 32-bit column c = elements 2c | 2c+1 of the row's K range), B through a descriptor
-__device__ __forceinline__ void mma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t hi, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      ".reg .b64 db;\n\t"
-      "mov.b64 db, {%2, %3};\n\t"
-      "setp.ne.b32 p, %5, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n\t"
-      "}" ::"r"(d_tmem), "r"(a_tmem), "r"(b_lo), "r"(hi), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t* r) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
-}
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
-      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
-        "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
-        "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31]) : "memory");
-}
+using namespace tc;
+
 __device__ __forceinline__ float ex2f(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // SWIZZLE_128B K-major descriptor halves: lo = start>>4 | LBO(1)<<16 ; hi = SBO(1024>>4) | version 1<<14 | SW128 (2)<<29
 __device__ __forceinline__ uint32_t desc_lo(uint32_t saddr) { return ((saddr >> 4) & 0x3FFFu) | (1u << 16); }
 constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);
@@ -142,35 +57,17 @@ __device__ __forceinline__ uint32_t idesc_f16(int N) {   // D=F32, A=B=F16, K-ma
 }
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
   uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
-      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]),
-        "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]),
-        "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld32_issue(taddr, r);
+  tmem_ld_wait();
 #pragma unroll
   for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
-      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]),
-        "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]),
-        "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
 }
 // 64 accumulator columns of this thread's lane: both loads in flight before the one wait
 __device__ __forceinline__ void tmem_ld64(uint32_t taddr, float* v) {
   uint32_t r[64];
-  tmem_ld32_nowait(taddr, r);
-  tmem_ld32_nowait(taddr + 32, r + 32);
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld32_issue(taddr, r);
+  tmem_ld32_issue(taddr + 32, r + 32);
+  tmem_ld_wait();
 #pragma unroll
   for (int i = 0; i < 64; ++i) v[i] = __uint_as_float(r[i]);
 }
@@ -199,7 +96,7 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
                     const __grid_constant__ CUtensorMap tmEk, const __grid_constant__ CUtensorMap tmEv) {
   extern __shared__ unsigned char smem_raw[];
   // aligned by pointer arithmetic on the __shared__ array: keeps the shared address space (LDS/STS, not generic LD/ST)
-  AttSmem& sm = *reinterpret_cast<AttSmem*>(smem_raw + ((1024u - (s_u32(smem_raw) & 1023u)) & 1023u));
+  AttSmem& sm = *reinterpret_cast<AttSmem*>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
   const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * BQ;
@@ -233,24 +130,21 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
   uint64_t* p_full = &sm.bars[32];       // [4], the 4 warps of the slot's group
 
   if (threadIdx.x == 0) {
-    bar_init(e_full, 1); bar_init(q_ready, 8); bar_init(r_full, 1); bar_init(pb_full, 4); bar_init(o_full, 1); bar_init(pv_all, 1);
+    mbar_init(e_full, 1); mbar_init(q_ready, 8); mbar_init(r_full, 1); mbar_init(pb_full, 4); mbar_init(o_full, 1); mbar_init(pv_all, 1);
     for (int i = 0; i < NSTG; ++i) {
-      bar_init(&k_full[i], 1); bar_init(&k_empty[i], 1); bar_init(&s_full[i], 1); bar_init(&pv_done[i], 1); bar_init(&p_full[i], 4);
+      mbar_init(&k_full[i], 1); mbar_init(&k_empty[i], 1); mbar_init(&s_full[i], 1); mbar_init(&pv_done[i], 1); mbar_init(&p_full[i], 4);
     }
-    for (int i = 0; i < NSTV; ++i) { bar_init(&v_full[i], 1); bar_init(&v_empty[i], 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    for (int i = 0; i < NSTV; ++i) { mbar_init(&v_full[i], 1); mbar_init(&v_empty[i], 1); }
+    fence_mbarrier_init();
+    fence_proxy_async();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s_u32(&sm.tmem_slot)), "r"(TM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(&sm.tmem_slot, TM_COLS);
   // zero the Pband tile (generic proxy) before anybody can use it
   for (int idx = threadIdx.x; idx < BQ * 8; idx += kThreadsAtt) reinterpret_cast<uint4*>(sm.pband)[idx] = make_uint4(0, 0, 0, 0);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  fence_before();
+  fence_proxy_async();
+  tc_fence_before();
   __syncthreads();
-  fence_after();
+  tc_fence_after();
   const uint32_t tmem = sm.tmem_slot;
 
   if (warp == 0) {
@@ -258,24 +152,24 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
     // lane 0 streams the relative tables and the K tiles, lane 1 the V tiles: two independent rings, so that a full V ring
     // never holds back the K tile the next Q K^T is waiting for
     if (lane == 0) {
-      bar_expect(e_full, 2 * 32 * 128 + DKV * 128);
-      for (int kb = 0; kb < 2; ++kb) tma2(sm.ek[kb], &tmEk, kb * 64, 0, e_full);
-      tma2(sm.evt, &tmEv, 0, 0, e_full);
+      mbar_expect_tx(e_full, 2 * 32 * 128 + DKV * 128);
+      for (int kb = 0; kb < 2; ++kb) tma_load_2d(sm.ek[kb], &tmEk, kb * 64, 0, e_full);
+      tma_load_2d(sm.evt, &tmEv, 0, 0, e_full);
       int ks = 0;
       uint32_t kp = 1;
       for (int it = 0; it < ntiles; ++it) {
-        bar_wait(&k_empty[ks], kp);
-        bar_expect(&k_full[ks], 2 * BKV * 128);
-        for (int kb = 0; kb < 2; ++kb) tma3(sm.k[ks][kb], &tmK, a.n_heads * DKP + h * DKP + kb * 64, it * BKV, b, &k_full[ks]);
+        mbar_wait(&k_empty[ks], kp);
+        mbar_expect_tx(&k_full[ks], 2 * BKV * 128);
+        for (int kb = 0; kb < 2; ++kb) tma_load_3d(sm.k[ks][kb], &tmK, a.n_heads * DKP + h * DKP + kb * 64, it * BKV, b, &k_full[ks]);
         if (++ks == NSTG) { ks = 0; kp ^= 1; }
       }
     } else if (lane == 1) {
       int vs = 0;
       uint32_t vp = 1;
       for (int t = 0; t < ntiles; ++t) {
-        bar_wait(&v_empty[vs], vp);
-        bar_expect(&v_full[vs], 2 * BKV * 128);
-        for (int db = 0; db < 2; ++db) tma3(sm.v[vs][db], &tmV, 2 * a.n_heads * DKP + h * DKP + db * 64, t * BKV, b, &v_full[vs]);
+        mbar_wait(&v_empty[vs], vp);
+        mbar_expect_tx(&v_full[vs], 2 * BKV * 128);
+        for (int db = 0; db < 2; ++db) tma_load_3d(sm.v[vs][db], &tmV, 2 * a.n_heads * DKP + h * DKP + db * 64, t * BKV, b, &v_full[vs]);
         if (++vs == NSTV) { vs = 0; vp ^= 1; }
       }
     }
@@ -284,33 +178,33 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
     const int g = warp == 1 ? 0 : 1;
     const uint32_t id_s = idesc_f16(BKV), id_r = idesc_f16(32);
     const uint32_t q_tm = tmem + TM_Q;                   // A operand: 8 columns per K = 16 step
-    bar_wait(q_ready, 0);
-    fence_after();
+    mbar_wait(q_ready, 0);
+    tc_fence_after();
     if (g == 0) {
-      bar_wait(e_full, 0);
-      if (elect1()) {   // R = Q Ek^T : K = 96 = 4 + 2 MMAs
+      mbar_wait(e_full, 0);
+      if (elect_one()) {   // R = Q Ek^T : K = 96 = 4 + 2 MMAs
         for (int ks = 0; ks < 6; ++ks)
-          mma_f16_ts(tmem + TM_R, q_tm + 8u * ks, desc_lo(s_u32(sm.ek[ks >> 2])) + 2u * (ks & 3), kDescHi, id_r, ks ? 1u : 0u);
-        commit(r_full);
+          tc_mma_f16_ts(tmem + TM_R, q_tm + 8u * ks, desc_lo(smem_u32(sm.ek[ks >> 2])) + 2u * (ks & 3), kDescHi, id_r, ks ? 1u : 0u);
+        tc_commit(r_full);
       }
       __syncwarp();
     }
     // key tile it = g + 2 n lands in slot g + 2 (n & 1)
-    const uint32_t k_lo[2] = {desc_lo(s_u32(sm.k[g][0])), desc_lo(s_u32(sm.k[g + 2][0]))};
+    const uint32_t k_lo[2] = {desc_lo(smem_u32(sm.k[g][0])), desc_lo(smem_u32(sm.k[g + 2][0]))};
     constexpr uint32_t kKb = (BKV * 128) >> 4;            // second k-block of a stage, in descriptor units
     const int mine = (ntiles - g + 1) / 2;
     auto issue_qk = [&](int n, int odd) {
       const int slot = g + 2 * odd;
-      bar_wait(&k_full[slot], ((uint32_t)n >> 1) & 1u);
-      bar_wait(&pv_done[slot], (((uint32_t)n >> 1) & 1u) ^ 1u);   // P V of the slot's previous tile has read its P
-      fence_after();
-      if (elect1()) {
+      mbar_wait(&k_full[slot], ((uint32_t)n >> 1) & 1u);
+      mbar_wait(&pv_done[slot], (((uint32_t)n >> 1) & 1u) ^ 1u);   // P V of the slot's previous tile has read its P
+      tc_fence_after();
+      if (elect_one()) {
 #pragma unroll
         for (int ks = 0; ks < 6; ++ks)
-          mma_f16_ts(tmem + TM_S + 64u * slot, q_tm + 8u * ks, k_lo[odd] + (ks < 4 ? 0u : kKb) + 2u * (ks & 3), kDescHi, id_s,
+          tc_mma_f16_ts(tmem + TM_S + 64u * slot, q_tm + 8u * ks, k_lo[odd] + (ks < 4 ? 0u : kKb) + 2u * (ks & 3), kDescHi, id_s,
                      ks ? 1u : 0u);
-        commit(&s_full[slot]);
-        commit(&k_empty[slot]);
+        tc_commit(&s_full[slot]);
+        tc_commit(&k_empty[slot]);
       }
       __syncwarp();
     };
@@ -324,36 +218,36 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
     // SBO = 1024 B between groups of 8 keys, LBO = 8192 B between the two 64-channel blocks); N = 96 takes the first
     // block and half of the second.  No transposed copy of V.
     const uint32_t id_o = idesc_f16(DKV), id_ov = id_o | (1u << 16);
-    bar_wait(e_full, 0);                                 // Ev^T
+    mbar_wait(e_full, 0);                                 // Ev^T
     int vs_ = 0;
     uint32_t vp = 0;
     for (int it = 0; it < ntiles; ++it) {
       const int slot = it & 3;
-      bar_wait(&p_full[slot], ((uint32_t)it >> 2) & 1u); // probabilities of this tile are in tensor memory
-      bar_wait(&v_full[vs_], vp);
-      fence_after();
-      if (elect1()) {
+      mbar_wait(&p_full[slot], ((uint32_t)it >> 2) & 1u); // probabilities of this tile are in tensor memory
+      mbar_wait(&v_full[vs_], vp);
+      tc_fence_after();
+      if (elect_one()) {
         const uint32_t p_tm = tmem + TM_S + 64u * slot;
-        const uint32_t v_lo = ((s_u32(sm.v[vs_][0]) >> 4) & 0x3FFFu) | ((uint32_t)((BKV * 128) >> 4) << 16);
+        const uint32_t v_lo = ((smem_u32(sm.v[vs_][0]) >> 4) & 0x3FFFu) | ((uint32_t)((BKV * 128) >> 4) << 16);
         const uint32_t o_tm = tmem + TM_O + 96u * (it & 1);      // the group's own accumulator
 #pragma unroll
         for (int ks = 0; ks < BKV / 16; ++ks)
-          mma_f16_ts(o_tm, p_tm + 8u * ks, v_lo + 128u * ks, kDescHi, id_ov, (it > 1 || ks) ? 1u : 0u);   // 16 keys = 2048 B
-        commit(&pv_done[slot]);
-        commit(&v_empty[vs_]);
+          tc_mma_f16_ts(o_tm, p_tm + 8u * ks, v_lo + 128u * ks, kDescHi, id_ov, (it > 1 || ks) ? 1u : 0u);   // 16 keys = 2048 B
+        tc_commit(&pv_done[slot]);
+        tc_commit(&v_empty[vs_]);
       }
       __syncwarp();
       if (++vs_ == NSTV) { vs_ = 0; vp ^= 1; }
     }
-    if (elect1()) commit(pv_all);
+    if (elect_one()) tc_commit(pv_all);
     __syncwarp();
     // O_0 += Pband Ev  (K = 32: two MMAs, both operands in shared memory; O_0 and Pband are at the final scale)
-    bar_wait(pb_full, 0);
-    fence_after();
-    if (elect1()) {
-      const uint32_t p_lo = desc_lo(s_u32(sm.pband)), e_lo = desc_lo(s_u32(sm.evt));
-      for (int ks = 0; ks < 2; ++ks) mma_f16(tmem + TM_O, p_lo + 2u * ks, e_lo + 2u * ks, kDescHi, id_o, 1u);
-      commit(o_full);
+    mbar_wait(pb_full, 0);
+    tc_fence_after();
+    if (elect_one()) {
+      const uint32_t p_lo = desc_lo(smem_u32(sm.pband)), e_lo = desc_lo(smem_u32(sm.evt));
+      for (int ks = 0; ks < 2; ++ks) tc_mma_f16(tmem + TM_O, p_lo + 2u * ks, kDescHi, e_lo + 2u * ks, kDescHi, id_o, 1u);
+      tc_commit(o_full);
     }
     __syncwarp();
   } else {
@@ -379,20 +273,20 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
 #pragma unroll
       for (int c = 0; c < 3; ++c) tmem_st8(tmem + lane_base + TM_Q + grp * 24 + c * 8, qv + c * 8);
       tmem_st_wait();
-      fence_before();
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) bar_arrive(q_ready);
+      if (lane == 0) mbar_arrive(q_ready);
     }
     // relative-key logits of this row -> smem (dynamic indexing by key offset); written by the row's first warp
-    bar_wait(r_full, 0);
-    fence_after();
+    mbar_wait(r_full, 0);
+    tc_fence_after();
     if (grp == 0) {
       float rv[32];
       tmem_ld32(tmem + lane_base + TM_R, rv);
 #pragma unroll
       for (int r = 0; r < 24; ++r) sm.rtab[row * 24 + r] = rv[r];
     }
-    fence_before();
+    tc_fence_before();
     asm volatile("bar.sync 1, 256;" ::: "memory");      // the 8 softmax warps; R (= head of O_1) is dead from here on
     float m_run = -INFINITY, l_run = 0.f;
     const uint32_t o_addr = tmem + lane_base + TM_O + 96u * grp;
@@ -401,8 +295,8 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
       const int j0 = it * BKV;
       const int slot = grp + 2 * (n & 1);
       const uint32_t s_addr = tmem + lane_base + TM_S + 64u * slot;
-      bar_wait(&s_full[slot], ((uint32_t)n >> 1) & 1u);
-      fence_after();
+      mbar_wait(&s_full[slot], ((uint32_t)n >> 1) & 1u);
+      tc_fence_after();
       float s[BKV];
       tmem_ld64(s_addr, s);
       if (j0 <= q0 + BQ - 1 + a.window && j0 + BKV - 1 >= q0 - a.window) {
@@ -429,8 +323,8 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
         // raise the running max of the warp's rows; O_grp (settled once the group's previous P V has completed) follows
         const float m_new = fmaxf(m_run, m_t);
         if (n > 0) {
-          bar_wait(&pv_done[grp + 2 * ((n - 1) & 1)], ((uint32_t)(n - 1) >> 1) & 1u);
-          fence_after();
+          mbar_wait(&pv_done[grp + 2 * ((n - 1) & 1)], ((uint32_t)(n - 1) >> 1) & 1u);
+          tc_fence_after();
           const float sc = ex2f((m_run - m_new) * kLog2e);
           l_run *= sc;
 #pragma unroll
@@ -458,9 +352,9 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
       }
       tmem_st32(s_addr, pk);
       tmem_st_wait();
-      fence_before();
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) bar_arrive(&p_full[slot]);
+      if (lane == 0) mbar_arrive(&p_full[slot]);
     }
     // ---- combine the two groups: final row max / row sum, O_0 and the band probabilities at the final scale ----
     sm.xch[0][grp][row] = m_run;
@@ -473,8 +367,8 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
     const float f_o = n_o > 0 ? ex2f((m_o - m_fin) * kLog2e) : 0.f;
     const float lsum = l_run * f_me + l_o * f_o;
     if (grp == 0) {
-      bar_wait(pv_all, 0);
-      fence_after();
+      mbar_wait(pv_all, 0);
+      tc_fence_after();
 #pragma unroll
       for (int c0 = 0; c0 < DKV; c0 += 32) {
         float o[32];
@@ -491,13 +385,13 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
         const float pv = (j >= 0 && j < L) ? ex2f(fmaf(sm.rtab[row * 24 + r], kLog2e, -mb)) : 0.f;
         *reinterpret_cast<__half*>(sm.pband + row * 128 + (((r >> 3) ^ (row & 7)) << 4) + (r & 7) * 2) = __float2half_rn(pv);
       }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      fence_before();
+      fence_proxy_async();
+      tc_fence_before();
       __syncwarp();
-      if (lane == 0) bar_arrive(pb_full);
+      if (lane == 0) mbar_arrive(pb_full);
     }
-    bar_wait(o_full, 0);
-    fence_after();
+    mbar_wait(o_full, 0);
+    tc_fence_after();
     const bool valid = qi < L;
     const float inv = valid ? 1.f / lsum : 0.f;
     const float f1 = grp ? f_me : f_o;                  // scale of O_1 (O_0 is at the final scale already)
@@ -530,34 +424,9 @@ attention_tc_kernel(const AttArgs a, const __grid_constant__ CUtensorMap tmK, co
       }
     }
   }
-  fence_before();
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TM_COLS));
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn att_encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  }
-  return fn;
-}
-
-bool make_map(CUtensorMap* tm, const void* base, int rank, const cuuint64_t* dims, const cuuint64_t* strides,
-              const cuuint32_t* box) {
-  cuuint32_t es[3] = {1, 1, 1};
-  return att_encode_tiled()(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, rank, const_cast<void*>(base), dims, strides, box, es,
-                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  if (warp == 1) tmem_dealloc(tmem, TM_COLS);
 }
 
 }  // namespace
@@ -567,23 +436,26 @@ bool make_map(CUtensorMap* tm, const void* base, int rank, const cuuint64_t* dim
 cudaError_t launch_attention_tc(const void* qkv16, void* vt, const void* ek16, const void* evt16, const int* len, void* out,
                                 int B, int T, int n_heads, int dk, int window, cudaStream_t st) {
   if (dk != DKV || 2 * window + 1 > MAXREL || B <= 0 || T <= 0 || n_heads < 1) return cudaErrorInvalidValue;
-  if (!att_encode_tiled()) return cudaErrorNotSupported;
+  if (!tensor_map_encoder_available()) return cudaErrorNotSupported;
   const int ld = 3 * n_heads * DKP;
   (void)vt;   // the transposed copy of V is no longer made (the scratch argument stays in the ABI)
   CUtensorMap tmK, tmV, tmEk, tmEv;
   {
+    const CUtensorMapDataType f16 = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+    const CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B;
+    const CUtensorMapL2promotion l2 = CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
     cuuint64_t dims[3] = {(cuuint64_t)(2 * n_heads * DKP), (cuuint64_t)T, (cuuint64_t)B};   // only the q|k columns are visible
     cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)ld * 2 * (cuuint64_t)T};
     cuuint32_t boxk[3] = {64, BKV, 1};
-    if (!make_map(&tmK, qkv16, 3, dims, strides, boxk)) return cudaErrorInvalidValue;
+    if (!encode_tensor_map(&tmK, f16, 3, qkv16, dims, strides, boxk, sw, l2)) return cudaErrorInvalidValue;
     cuuint64_t vd[3] = {(cuuint64_t)ld, (cuuint64_t)T, (cuuint64_t)B};                        // the whole q|k|v row; keys >= T read as zero
-    if (!make_map(&tmV, qkv16, 3, vd, strides, boxk)) return cudaErrorInvalidValue;
+    if (!encode_tensor_map(&tmV, f16, 3, qkv16, vd, strides, boxk, sw, l2)) return cudaErrorInvalidValue;
     cuuint64_t ekd[2] = {DKP, 32}, eks[1] = {DKP * 2};
     cuuint32_t boxek[2] = {64, 32};
-    if (!make_map(&tmEk, ek16, 2, ekd, eks, boxek)) return cudaErrorInvalidValue;
+    if (!encode_tensor_map(&tmEk, f16, 2, ek16, ekd, eks, boxek, sw, l2)) return cudaErrorInvalidValue;
     cuuint64_t evd[2] = {64, DKP}, evs[1] = {64 * 2};
     cuuint32_t boxev[2] = {64, DKV};
-    if (!make_map(&tmEv, evt16, 2, evd, evs, boxev)) return cudaErrorInvalidValue;
+    if (!encode_tensor_map(&tmEv, f16, 2, evt16, evd, evs, boxev, sw, l2)) return cudaErrorInvalidValue;
   }
   const size_t smem = sizeof(AttSmem) + 1024;
   static SmemOptIn opt;

@@ -76,12 +76,8 @@ using namespace tc;
 __device__ __forceinline__ void epilogue_generic16(const TcConvDesc& p, uint32_t taddr, bool row_ok, bool valid, int b,
                                                    long long orow, int co, const float* sb, const float4* pre) {
   uint32_t r[16];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld16_issue(taddr, r);
+  tmem_ld_wait();
   if (!row_ok) return;
   const long long Lout = (long long)p.Lj * p.out_stride;
   float v[16];
@@ -204,15 +200,8 @@ __device__ __forceinline__ void epilogue_lean64(const TcConvDesc& p, uint32_t ta
                                                 int co, const float* sb, const float4* pre, bool have_pre) {
   uint32_t r[64];
 #pragma unroll
-  for (int q = 0; q < 4; ++q)
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[q * 16 + 0]), "=r"(r[q * 16 + 1]), "=r"(r[q * 16 + 2]), "=r"(r[q * 16 + 3]), "=r"(r[q * 16 + 4]),
-          "=r"(r[q * 16 + 5]), "=r"(r[q * 16 + 6]), "=r"(r[q * 16 + 7]), "=r"(r[q * 16 + 8]), "=r"(r[q * 16 + 9]),
-          "=r"(r[q * 16 + 10]), "=r"(r[q * 16 + 11]), "=r"(r[q * 16 + 12]), "=r"(r[q * 16 + 13]), "=r"(r[q * 16 + 14]),
-          "=r"(r[q * 16 + 15])
-        : "r"(taddr + 16u * q));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  for (int q = 0; q < 4; ++q) tmem_ld16_issue(taddr + 16u * q, r + q * 16);
+  tmem_ld_wait();
   if (!row_ok) return;
   const long long Lout = (long long)p.Lj * p.out_stride;
   float v[64];
@@ -361,16 +350,12 @@ conv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, cons
     for (int i = 0; i < NA; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 1); }
     for (int i = 0; i < NB; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], kEpiWarps / 2); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW)) : "memory");
+    fence_mbarrier_init();
+    fence_proxy_async();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmW);
   }
-  if (warp == 1) {  // TMEM: two accumulator buffers of N columns (power of two >= 32 in total)
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)p.tmem_cols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)p.tmem_cols);   // two accumulator buffers of N columns (power of two >= 32)
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -750,7 +735,7 @@ conv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, cons
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&acc_empty[eg])) : "memory");
+      if (lane == 0) mbar_arrive(&acc_empty[eg]);
     }
     if (p.tma_out && lane == 0) bulk_wait_all();    // staged stores complete before the CTA's smem goes away
   }
@@ -758,9 +743,7 @@ conv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, cons
   if (warp == 2 && lane == 0) trace_mark(6);                                // first epilogue warp done
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)p.tmem_cols));
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols);
 }
 
 constexpr size_t kStageBytes = 8 * 2 * 2048 + 1024;   // tma_out staging (+ alignment slack)
@@ -777,18 +760,15 @@ size_t tc_smem_bytes(const TcConvDesc& d) {
 }
 
 // ---- driver entry point for tensor-map encoding (no link-time dependency on libcuda) --------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+using EncodeTiledFn = decltype(&cuTensorMapEncodeTiled);
 EncodeTiledFn encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
+  static const EncodeTiledFn fn = [] {
     void* ptr = nullptr;
     cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  }
+    const bool found = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
+                       qres == cudaDriverEntryPointSuccess;
+    return found ? reinterpret_cast<EncodeTiledFn>(ptr) : nullptr;
+  }();
   return fn;
 }
 
@@ -1115,6 +1095,17 @@ inline unsigned grid_for(long long total, int threads) {
 
 }  // namespace
 
+bool tensor_map_encoder_available() { return encode_tiled() != nullptr; }
+
+bool encode_tensor_map(CUtensorMap* tm, CUtensorMapDataType dt, int rank, const void* base, const cuuint64_t* dims,
+                       const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle,
+                       CUtensorMapL2promotion l2) {
+  const EncodeTiledFn enc = encode_tiled();
+  const cuuint32_t elem_strides[5] = {1, 1, 1, 1, 1};
+  return enc && enc(tm, dt, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, elem_strides,
+                    CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 cudaError_t conv_tc_set_trace(void* buf) {
   unsigned long long* p = reinterpret_cast<unsigned long long*>(buf);
   return cudaMemcpyToSymbol(g_trace, &p, sizeof(p));
@@ -1128,8 +1119,7 @@ cudaError_t launch_conv_tc(const TcConvDesc& d_in, int B, cudaStream_t st) {
       (d.tap_w > 0 && (d.ntaps % d.tap_w != 0 || d.dil2 < (d.tap_w - 1) * d.dil)) || d.pad_period < 0 || (d.pad_period > 0 && !d.generic) || (d.accum && !d.y32) || B <= 0 || !d.x16 || !d.w16 ||
       d.a_fp16 || (d.res16 && d.res32) || (d.acc_f16 && (d.generic || d.Cout_total % 8)) || !tc_div_exact(d.div))
     return cudaErrorInvalidValue;
-  EncodeTiledFn enc = encode_tiled();
-  if (!enc) return cudaErrorNotSupported;
+  if (!tensor_map_encoder_available()) return cudaErrorNotSupported;
   {
     static const int lean_on = [] { const char* e = getenv("RVCB200_LEAN_EPI"); return e ? atoi(e) : 1; }();
     d.reserved1 = lean_on ? 0 : 1;
@@ -1211,16 +1201,14 @@ cudaError_t launch_conv_tc(const TcConvDesc& d_in, int B, cudaStream_t st) {
     const cuuint64_t ldx = (cuuint64_t)(d.generic && d.ldx16 ? d.ldx16 : d.Cin);
     cuuint64_t strides[2] = {ldx * 2, ldx * 2 * (cuuint64_t)d.L_in};
     cuuint32_t box[3] = {(cuuint32_t)KBLK, (cuuint32_t)R, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    if (enc(&tmA, dt, 3, const_cast<void*>(d.x16), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmA, dt, 3, d.x16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
     const cuuint64_t wrows = (cuuint64_t)d.G * n_nt * d.ntaps * nkb * d.N;
     cuuint64_t wdims[2] = {(cuuint64_t)KBLK, wrows};
     cuuint64_t wstrides[1] = {(cuuint64_t)KBLK * 2};
     cuuint32_t wbox[2] = {(cuuint32_t)KBLK, (cuuint32_t)d.N};
-    if (enc(&tmW, dt, 2, const_cast<void*>(d.w16), wdims, wstrides, wbox, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmW, dt, 2, d.w16, wdims, wstrides, wbox, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
   }
   tmY = tmA;
@@ -1229,10 +1217,8 @@ cudaError_t launch_conv_tc(const TcConvDesc& d_in, int B, cudaStream_t st) {
     cuuint64_t ostr[3] = {(cuuint64_t)d.Cout_total * 2, (cuuint64_t)d.Cout_total * 2 * d.out_stride,
                           (cuuint64_t)d.Cout_total * 2 * d.out_stride * (cuuint64_t)d.Lj};
     cuuint32_t obox[4] = {32, 1, 32, 1};
-    cuuint32_t oes[4] = {1, 1, 1, 1};
-    if (enc(&tmY, d.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, d.y16, odims, ostr, obox, oes,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmY, d.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, d.y16, odims,
+                           ostr, obox, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
       return cudaErrorInvalidValue;
   }
   static SmemOptIn opt_s, opt_g;

@@ -1,5 +1,6 @@
 // Descriptor + launchers of the tcgen05 convolution path (see conv_tc.cu).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 
 #include "../../include/rvcb200.h"
@@ -7,6 +8,15 @@
 namespace rvc {
 
 typedef rvcb200_tc_conv_desc TcConvDesc;
+
+// TMA tensor maps of the tcgen05 kernels, encoded by the driver's cuTensorMapEncodeTiled (looked up once through the
+// runtime, so the library does not link libcuda).  False when the driver does not provide it.
+bool tensor_map_encoder_available();
+// One tiled tensor map with unit element strides, no interleave and the zero out-of-bounds fill (loads read elements
+// outside `dims` as zero, stores skip them); false when encoding fails.
+bool encode_tensor_map(CUtensorMap* tm, CUtensorMapDataType dt, int rank, const void* base, const cuuint64_t* dims,
+                       const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapSwizzle swizzle,
+                       CUtensorMapL2promotion l2);
 
 constexpr int kPadF = 32;                                   // zero rows in front of every PV plane
 inline int pv_pitch_rows(long long L) { return (int)(((L + 127) / 128) * 128 + 128); }   // Lp

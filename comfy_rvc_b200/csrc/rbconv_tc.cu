@@ -125,16 +125,12 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
     for (int i = 0; i < K::NB; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 4); }
     for (int i = 0; i < 16; ++i) mbar_init(&res_full[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW)) : "memory");
+    fence_mbarrier_init();
+    fence_proxy_async();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmW);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)K::TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)K::TMEM_COLS);
   for (int i = threadIdx.x; i < C; i += kRbThreads) sbias[i] = p.bias[i];
   if (p.inj_har) {
     const int nw = p.inj_k * p.inj_cn;
@@ -321,19 +317,11 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
           const bool row_ok = row < p.Lj;
           if (do_acc && ci + 1 < K::NCH) load_acc(ci + 1, u ^ 1);
           uint32_t r[32];
-          const uint32_t taddr = tbase + (uint32_t)(ms * C + c0);
-          asm volatile(
-              "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
-              "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-              : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-                "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-                "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-                "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-              : "r"(taddr));
+          tmem_ld32_issue(tbase + (uint32_t)(ms * C + c0), r);
           float4 bq[8];                               // bias: its smem latency hides under the TMEM load
 #pragma unroll
           for (int k4 = 0; k4 < 8; ++k4) bq[k4] = lds_f4(sbias + c0 + k4 * 4);
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+          tmem_ld_wait();
           if (tanh_out) {                             // (warp-uniform) the 128 B a warp stores are contiguous
             if (c0 == 0 && row_ok) tanh_out[(size_t)b * (size_t)p.Lj + row] = tanhf(__uint_as_float(r[0]) + bq[0].x);
             continue;
@@ -434,53 +422,33 @@ rbconv_tc_kernel(const TcConvDesc p, const __grid_constant__ CUtensorMap tmA, co
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&acc_empty[eg])) : "memory");
+      if (lane == 0) mbar_arrive(&acc_empty[eg]);
     }
     if (lane == 0) bulk_wait_all();     // staged stores complete before the CTA's smem goes away
   }
   // ------------------------------------ teardown -------------------------------------------------
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)K::TMEM_COLS));
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn rb_encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  }
-  return fn;
+  if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)K::TMEM_COLS);
 }
 
 template <int C, int NTAPS, int DIL, int MSUB>
 cudaError_t launch_one(const TcConvDesc& d, int B, cudaStream_t st) {
   using K = RbCfg<C, NTAPS, DIL, MSUB>;
-  EncodeTiledFn enc = rb_encode_tiled();
-  if (!enc) return cudaErrorNotSupported;
+  if (!tensor_map_encoder_available()) return cudaErrorNotSupported;
   CUtensorMap tmA, tmW, tmR, tmY;
   const CUtensorMapDataType dt = d.in_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  cuuint32_t es[3] = {1, 1, 1};
   {
     cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)d.L_in, (cuuint64_t)B};
     cuuint64_t strides[2] = {(cuuint64_t)C * 2, (cuuint64_t)C * 2 * (cuuint64_t)d.L_in};
     cuuint32_t box[3] = {64, (cuuint32_t)K::RB, 1};
-    if (enc(&tmA, dt, 3, const_cast<void*>(d.x16), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmA, dt, 3, d.x16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
     cuuint64_t wdims[2] = {64, (cuuint64_t)NTAPS * K::NKB * C};
     cuuint64_t wstrides[1] = {128};
     cuuint32_t wbox[2] = {64, (cuuint32_t)C};
-    if (enc(&tmW, dt, 2, const_cast<void*>(d.w16), wdims, wstrides, wbox, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmW, dt, 2, d.w16, wdims, wstrides, wbox, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
     // epilogue boxes: [32 rows][32 channels] of the 16-bit channels-last residual / output, SWIZZLE_64B staging
     tmR = tmA;
@@ -488,15 +456,11 @@ cudaError_t launch_one(const TcConvDesc& d, int B, cudaStream_t st) {
     cuuint64_t odims[3] = {(cuuint64_t)C, (cuuint64_t)d.Lj, (cuuint64_t)B};
     cuuint64_t ostrides[2] = {(cuuint64_t)C * 2, (cuuint64_t)C * 2 * (cuuint64_t)d.Lj};
     cuuint32_t obox[3] = {32, 32, 1};
-    if (d.res16 &&
-        enc(&tmR, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(d.res16), odims, ostrides, obox, es,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (d.res16 && !encode_tensor_map(&tmR, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, d.res16, odims, ostrides, obox,
+                                      CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
       return cudaErrorInvalidValue;
-    if (d.y16 &&
-        enc(&tmY, d.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, d.y16, odims, ostrides,
-            obox, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (d.y16 && !encode_tensor_map(&tmY, d.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3,
+                                    d.y16, odims, ostrides, obox, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
       return cudaErrorInvalidValue;
   }
   static SmemOptIn opt;

@@ -141,22 +141,6 @@ __device__ __forceinline__ void ring_next(Ring& r) {
   if (++r.i == (uint32_t)N) { r.i = 0; r.ph ^= 1u; }
 }
 
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
-      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
 template <int C, int NTAPS, int DIL, int VAR>
 __global__ void __launch_bounds__(pair_threads(pair_sel(C, NTAPS, VAR).e1g, pair_sel(C, NTAPS, VAR).e2g), 1)
 rbpair_tc_kernel(const PairParams p, const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW1,
@@ -199,17 +183,13 @@ rbpair_tc_kernel(const PairParams p, const __grid_constant__ CUtensorMap tmA, co
     for (int i = 0; i < NB1; ++i) { mbar_init(&acc1_full[i], 1); mbar_init(&acc1_empty[i], 4); }
     for (int i = 0; i < 2; ++i) { mbar_init(&acc2_full[i], 1); mbar_init(&acc2_empty[i], 4); }
     for (int i = 0; i < NH; ++i) { mbar_init(&h_full[i], 4); mbar_init(&h_empty[i], 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmA)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW1)) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(&tmW2)) : "memory");
+    fence_mbarrier_init();
+    fence_proxy_async();
+    prefetch_tmap(&tmA);
+    prefetch_tmap(&tmW1);
+    prefetch_tmap(&tmW2);
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"((uint32_t)K::TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 1) tmem_alloc(tmem_slot, (uint32_t)K::TMEM_COLS);
   for (int i = threadIdx.x; i < C; i += K::THREADS) { sbias1[i] = p.bias1[i]; sbias2[i] = p.bias2[i]; }
   // rows [TILE_M, H_ROWS) of an h tile are only ever read for output rows that are discarded; keep them finite
   for (int i = threadIdx.x; i < (int)((size_t)NH * K::H_BYTES / 16); i += K::THREADS)
@@ -533,51 +513,31 @@ rbpair_tc_kernel(const PairParams p, const __grid_constant__ CUtensorMap tmA, co
   // ------------------------------------ teardown -------------------------------------------------
   tc_fence_before();
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)K::TMEM_COLS));
-  }
-}
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn pair_encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  }
-  return fn;
+  if (warp == 1) tmem_dealloc(tmem_base, (uint32_t)K::TMEM_COLS);
 }
 
 template <int C, int NTAPS, int DIL, int VAR>
 cudaError_t launch_pair_one(const TcConvDesc& d1, const TcConvDesc& d2, int B, cudaStream_t st) {
   using K = PairCfg<C, NTAPS, DIL, VAR>;
-  EncodeTiledFn enc = pair_encode_tiled();
-  if (!enc) return cudaErrorNotSupported;
+  if (!tensor_map_encoder_available()) return cudaErrorNotSupported;
   CUtensorMap tmA, tmW1, tmW2, tmY, tmYt;
   const CUtensorMapDataType dt1 = d1.in_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
   const CUtensorMapDataType dt2 = d2.in_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
-  cuuint32_t es[3] = {1, 1, 1};
   const int L = d1.Lj;
   {
     cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)L, (cuuint64_t)B};
     cuuint64_t strides[2] = {(cuuint64_t)C * 2, (cuuint64_t)C * 2 * (cuuint64_t)L};
     cuuint32_t box[3] = {64, (cuuint32_t)K::RB, 1};
-    if (enc(&tmA, dt1, 3, const_cast<void*>(d1.x16), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmA, dt1, 3, d1.x16, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
     cuuint64_t wdims[2] = {64, (cuuint64_t)NTAPS * C};
     cuuint64_t wstrides[1] = {128};
     cuuint32_t wbox[2] = {64, (cuuint32_t)C};
-    if (enc(&tmW1, dt1, 2, const_cast<void*>(d1.w16), wdims, wstrides, wbox, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmW1, dt1, 2, d1.w16, wdims, wstrides, wbox, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
-    if (enc(&tmW2, dt2, 2, const_cast<void*>(d2.w16), wdims, wstrides, wbox, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    if (!encode_tensor_map(&tmW2, dt2, 2, d2.w16, wdims, wstrides, wbox, CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
       return cudaErrorInvalidValue;
     tmY = tmA;
     tmYt = tmA;
@@ -585,11 +545,9 @@ cudaError_t launch_pair_one(const TcConvDesc& d1, const TcConvDesc& d2, int B, c
       const CUtensorMapDataType dto = d2.out_bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
       cuuint32_t obox[3] = {32, 32, 1};
       cuuint32_t tbox[3] = {32, (cuuint32_t)K::TAIL_ROWS, 1};
-      if (enc(&tmY, dto, 3, d2.y16, dims, strides, obox, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+      if (!encode_tensor_map(&tmY, dto, 3, d2.y16, dims, strides, obox, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
         return cudaErrorInvalidValue;
-      if (enc(&tmYt, dto, 3, d2.y16, dims, strides, tbox, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
-              CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+      if (!encode_tensor_map(&tmYt, dto, 3, d2.y16, dims, strides, tbox, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
         return cudaErrorInvalidValue;
     }
   }

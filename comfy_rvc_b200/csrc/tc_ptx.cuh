@@ -1,5 +1,6 @@
-// PTX wrappers (mbarrier, TMA, tcgen05) and the lean decoder epilogue shared by the tcgen05 convolution kernels
-// (conv_tc.cu: generic persistent implicit-GEMM conv; rbconv_tc.cu: compile-time specialised resblock conv).
+// PTX wrappers (mbarrier, TMA, tcgen05) of every tcgen05 kernel -- conv_tc.cu (generic persistent implicit-GEMM conv),
+// rbconv_tc.cu (compile-time specialised resblock conv), rbpair_tc.cu (fused resblock pair), attention_tc.cu (windowed
+// attention) -- and the epilogue helpers of the three convolution kernels.
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -19,6 +20,10 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void fence_mbarrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   const uint32_t addr = smem_u32(bar);
   uint32_t done;
@@ -42,6 +47,9 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* tm, in
       "cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
+}
+__device__ __forceinline__ void prefetch_tmap(const CUtensorMap* tm) {
+  asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tm)) : "memory");
 }
 __device__ __forceinline__ bool elect_one() {   // one lane of a converged warp (elect.sync)
   uint32_t pred;
@@ -94,6 +102,63 @@ __device__ __forceinline__ void tc_commit_pred(uint64_t* bar, uint32_t leader) {
       "@q tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t"
       "}" ::"r"(smem_u32(bar)), "r"(leader) : "memory");
 }
+// A operand in tensor memory (lane = row, 32-bit column c = elements 2c | 2c+1 of the row's K range), B through a descriptor
+__device__ __forceinline__ void tc_mma_f16_ts(uint32_t d_tmem, uint32_t a_tmem, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
+                                              uint32_t acc) {
+  asm volatile(
+      "{\n\t"
+      ".reg .pred p;\n\t"
+      ".reg .b64 db;\n\t"
+      "mov.b64 db, {%2, %3};\n\t"
+      "setp.ne.b32 p, %5, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %4, p;\n\t"
+      "}" ::"r"(d_tmem), "r"(a_tmem), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc) : "memory");
+}
+
+// ---- tensor memory: allocation (one warp), loads and stores of this thread's lane ----
+// writes the base address to *slot and gives up the right to allocate more, so that the next CTA on the SM may
+__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t cols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(cols));
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols));
+}
+// r[0..32) / r[0..16) = columns [taddr, +32) / [taddr, +16); the registers are valid only after tmem_ld_wait(), so that
+// other loads can be issued in between
+__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t* r) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
+      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
+        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
+        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+      : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_ld16_issue(uint32_t taddr, uint32_t* r) {
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+      : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t* r) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
+               ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]) : "memory");
+}
+__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t* r) {
+  asm volatile(
+      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
+      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31,%32};"
+      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
+        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
+        "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
+        "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31]) : "memory");
+}
+__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
 // K-major SWIZZLE_128B shared-memory descriptor (cute/arch/mma_sm100_desc.hpp SmemDescriptor):
 // start>>4 [0,14) | LBO>>4 [16,30) (unused for swizzled K-major, 1) | SBO>>4 [32,46) = 1024 B |
 // version 1 [46,48) | base_offset [49,52) | layout_type SWIZZLE_128B = 2 [61,64)
@@ -183,23 +248,8 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvDesc& p, uint32_t tad
                                                const unsigned char* r16row = nullptr, unsigned char* stage_row = nullptr,
                                                uint32_t sw_x = 0) {
   uint32_t r[CH];
-  if (CH == 32) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
-        "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16 % CH]),
-          "=r"(r[17 % CH]), "=r"(r[18 % CH]), "=r"(r[19 % CH]), "=r"(r[20 % CH]), "=r"(r[21 % CH]), "=r"(r[22 % CH]),
-          "=r"(r[23 % CH]), "=r"(r[24 % CH]), "=r"(r[25 % CH]), "=r"(r[26 % CH]), "=r"(r[27 % CH]), "=r"(r[28 % CH]),
-          "=r"(r[29 % CH]), "=r"(r[30 % CH]), "=r"(r[31 % CH])
-        : "r"(taddr));
-  } else {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-  }
+  if constexpr (CH == 32) tmem_ld32_issue(taddr, r);
+  else tmem_ld16_issue(taddr, r);
   float4 rr[CH / 4], aa[CH / 4];
   uint4 rh[CH / 8];
   if (row_ok) {
@@ -231,7 +281,7 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvDesc& p, uint32_t tad
       }
     }
   }
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+  tmem_ld_wait();
   if (!row_ok) return;
   float v[CH];
 #pragma unroll
