@@ -128,6 +128,10 @@ SYMBOLS = {
                                            C.c_int32, C.c_float, C.c_int32, C.c_void_p]),
     "rvcb200_op_absmax": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p]),
     "rvcb200_op_to_int16": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rvcb200_op_rms_halfblock": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "rvcb200_op_rms_fold": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
+    "rvcb200_op_rms_gain": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                      C.c_double, C.c_void_p]),
     "rvcb200_op_hubert_conv0": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                           C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int64, C.c_void_p]),
     "rvcb200_op_layernorm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,

@@ -126,6 +126,10 @@ cudaError_t launch_prepare_feats(const void* f, const void* f0, int dtype, const
                                  float protect, int use_protect, cudaStream_t st);
 cudaError_t launch_absmax(const float* x, long long n, float* out, int reset, cudaStream_t st);
 cudaError_t launch_to_int16(const float* x, long long n, const float* absmax, short* out, cudaStream_t st);
+cudaError_t launch_rms_halfblock(const void* x, int x_f64, long long len, long long offset, int hop, double* out, cudaStream_t st);
+cudaError_t launch_rms_fold(const double* table, int rows, long long n_hb, int frame_length, float* rms, cudaStream_t st);
+cudaError_t launch_rms_gain(float* x, long long len, long long offset, long long N, const float* rms1, long long n1, const float* rms2,
+                            long long n2, double rate, cudaStream_t st);
 cudaError_t launch_quiet_point(const double* audio_pad, long long lo, long long hi, int window, double* best_v, long long* best_j,
                                int n_blocks, cudaStream_t st);
 

@@ -1186,6 +1186,25 @@ int rvcb200_op_to_int16(const float* x, int64_t n, const float* absmax, int16_t*
   return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
 }
 
+// change_rms (lib/model_utils.py:39, vc_infer_pipeline.py:183): float32 squares summed in double, in a grid-independent order.
+int rvcb200_op_rms_halfblock(const void* x, int32_t x_f64, int64_t len, int64_t offset, int32_t hop, double* out, void* stream) {
+  cudaError_t e = launch_rms_halfblock(x, x_f64, len, offset, hop, out, reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
+// change_rms (lib/model_utils.py:39, vc_infer_pipeline.py:183): rows folded in order in double, mean rounded once to float32.
+int rvcb200_op_rms_fold(const double* table, int32_t rows, int64_t n_hb, int32_t frame_length, float* rms, void* stream) {
+  cudaError_t e = launch_rms_fold(table, rows, n_hb, frame_length, rms, reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
+// change_rms (lib/model_utils.py:39, vc_infer_pipeline.py:183): torch's float32 linear interpolation, powf, two float32 products.
+int rvcb200_op_rms_gain(float* x, int64_t len, int64_t offset, int64_t N, const float* rms1, int64_t n1, const float* rms2, int64_t n2,
+                        double rate, void* stream) {
+  cudaError_t e = launch_rms_gain(x, len, offset, N, rms1, n1, rms2, n2, rate, reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
 int rvcb200_op_hubert_conv0(const float* x, const float* w, const float* gn_w, const float* gn_b, double* stats, void* y16,
                             int32_t B, int64_t n, int32_t C, int32_t K, int32_t S, float eps, int64_t y_bstride, void* stream) {
   cudaError_t e = launch_hubert_conv0(x, w, gn_w, gn_b, stats, y16, B, n, C, K, S, eps, y_bstride,

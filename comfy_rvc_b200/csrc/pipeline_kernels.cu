@@ -2,9 +2,12 @@
 //   prepare_feats : x2 nearest interpolation of the HuBERT frames + "protect" blend   (vc_infer_pipeline.py:77-95)
 //   absmax        : max |x| over the concatenated song                                 (vc_infer_pipeline.py:188)
 //   to_int16      : x * 32768 / (max / 0.99), C truncation                             (vc_infer_pipeline.py:188-189)
-// All three are HBM-bound streaming kernels (one pass, 16-byte accesses); they exist so that a whole song is
+//   rms_halfblock / rms_fold / rms_gain : the volume-envelope mix `change_rms`      (lib/model_utils.py:39, :183)
+// All of them are HBM-bound streaming kernels (one pass, 16-byte accesses); they exist so that a whole song is
 // converted without a host round trip per segment (the reference syncs and gc's after every segment, :102-112).
 #include <cuda_fp16.h>
+
+#include <cmath>
 
 #include "common.cuh"
 
@@ -119,6 +122,82 @@ __global__ void quiet_point_kernel(const double* __restrict__ a, long long lo, l
   if (threadIdx.x == 0) { best_v[blockIdx.x] = sv[0]; best_j[blockIdx.x] = sj[0]; }
 }
 
+// ---- volume-envelope mix (change_rms, lib/model_utils.py:39, called at vc_infer_pipeline.py:183) ----------------------------
+// librosa.feature.rms(frame_length = 2 * hop, center=True, pad_mode="constant"): frame f covers half-blocks f - 1 and f, where
+// half-block b is samples [b * hop, (b + 1) * hop) of the signal and half-blocks outside it are zero.  So the envelope is
+// built from half-block sums, which a piece of the signal (one segment's output) can contribute to on its own.
+
+// One block per half-block the piece touches: out[k] = sum over the piece's samples of half-block offset / hop + k of
+// float32(x)^2 (the square rounded to float32 like numpy's `np.power(x, 2, dtype=np.float32)`), accumulated in double.
+// Thread t adds the samples at global positions b * hop + t + 256 j in ascending j; a fixed tree then combines the 256
+// threads.  The order depends only on which samples of the half-block the piece holds, not on the grid or the piece's
+// global offset, so every rank produces the same bits for the same piece.
+template <typename T>
+__global__ void __launch_bounds__(256) rms_halfblock_kernel(const T* __restrict__ x, long long len, long long offset, int hop,
+                                                            double* __restrict__ out) {
+  const long long b = offset / hop + blockIdx.x;
+  const long long glo = b * hop > offset ? b * hop : offset;                       // global sample range of this block
+  const long long ghi = (b + 1) * hop < offset + len ? (b + 1) * hop : offset + len;
+  long long g = b * hop + threadIdx.x;
+  if (g < glo) g += (glo - g + blockDim.x - 1) / blockDim.x * blockDim.x;
+  double acc = 0.0;
+#pragma unroll 4
+  for (; g < ghi; g += blockDim.x) {
+    const float v = (float)x[g - offset];                                           // float64 input: rounded to nearest
+    acc = __dadd_rn(acc, (double)__fmul_rn(v, v));
+  }
+  __shared__ double sm[256];
+  sm[threadIdx.x] = acc;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) sm[threadIdx.x] = __dadd_rn(sm[threadIdx.x], sm[threadIdx.x + o]);
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
+}
+
+// rms[f] = sqrt(mean of frame f) in float32, f < n_hb.  table[r][b] (r < rows, row stride n_hb) holds half-block sums split
+// over rows (one row per segment, zero where a segment does not reach); the rows are added in ascending order from +0.0,
+// then frame f = hb[f - 1] + hb[f] (hb[-1] = 0), divided by frame_length in double and rounded once to float32.
+__global__ void rms_fold_kernel(const double* __restrict__ table, int rows, long long n_hb, int frame_length, float* __restrict__ rms) {
+  for (long long f = (long long)blockIdx.x * blockDim.x + threadIdx.x; f < n_hb; f += (long long)gridDim.x * blockDim.x) {
+    double a = 0.0, b = 0.0;
+    for (int r = 0; r < rows; ++r) {
+      if (f > 0) a = __dadd_rn(a, table[(long long)r * n_hb + f - 1]);
+      b = __dadd_rn(b, table[(long long)r * n_hb + f]);
+    }
+    rms[f] = __fsqrt_rn(__double2float_rn(__ddiv_rn(__dadd_rn(a, b), (double)frame_length)));
+  }
+}
+
+// F.interpolate(env[1][1][n_in], size=N, mode="linear", align_corners=False)[d] exactly as torch's float32 CPU kernel
+// rounds it: the source index is one fused multiply-add on float32(d) + 0.5 (with N > 2^24 that sum already rounds), and
+// the blend is fma(x0, 1 - lam, x1 * lam).  Explicit intrinsics: a more accurate index misses torch by up to 9 % at N = 86.4 M.
+__device__ __forceinline__ float interp_linear(const float* __restrict__ env, int n_in, float scale, long long d) {
+  const float t = __fadd_rn(__ll2float_rn(d), 0.5f);
+  const float src = fmaxf(__fmaf_rn(t, scale, -0.5f), 0.f);
+  const int i0 = min((int)src, n_in - 1);
+  const int i1 = min(i0 + 1, n_in - 1);
+  const float lam = fminf(fmaxf(__fsub_rn(src, (float)i0), 0.f), 1.f);
+  return __fmaf_rn(env[i0], __fsub_rn(1.f, lam), __fmul_rn(env[i1], lam));
+}
+
+// x[i] *= pow(e1, 1 - rate) * pow(max(e2, 1e-6), rate - 1) for the samples d = offset + i of a song of N samples:
+// e1 / e2 = the input / output envelopes interpolated to N; the exponents are float32(1 - rate) and float32(rate - 1)
+// (`torch.tensor(1 - rate)`); the product and the update are single float32 roundings (torch's `*`, numpy's `*=`).
+__global__ void rms_gain_kernel(float* __restrict__ x, long long len, long long offset, long long N, const float* __restrict__ e1, int n1,
+                                const float* __restrict__ e2, int n2, float p1, float p2) {
+  const float fN = __ll2float_rn(N);
+  const float s1 = __fdiv_rn((float)n1, fN), s2 = __fdiv_rn((float)n2, fN);
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < len; i += (long long)gridDim.x * blockDim.x) {
+    const long long d = offset + i;
+    const float v1 = interp_linear(e1, n1, s1, d);
+    const float v2 = fmaxf(interp_linear(e2, n2, s2, d), 1e-6f);
+    const float gain = __fmul_rn(powf(v1, p1), powf(v2, p2));
+    x[i] = __fmul_rn(x[i], gain);
+  }
+}
+
 inline unsigned stream_grid(long long work, int threads) {
   long long blocks = (work + threads - 1) / threads;
   const long long cap = 148 * 8;
@@ -165,6 +244,38 @@ cudaError_t launch_to_int16(const float* x, long long n, const float* absmax, sh
   if (n < 0 || (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(out) & 7)) return cudaErrorInvalidValue;
   if (n == 0) return cudaSuccess;
   to_int16_kernel<<<stream_grid(n / 4 + 1, 256), 256, 0, st>>>(x, n, absmax, out);
+  launch_counter().n++;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rms_halfblock(const void* x, int x_f64, long long len, long long offset, int hop, double* out, cudaStream_t st) {
+  if (!x || !out || len < 0 || offset < 0 || hop < 1 || (x_f64 != 0 && x_f64 != 1)) return cudaErrorInvalidValue;
+  if (len == 0) return cudaSuccess;
+  const long long blocks = (offset + len - 1) / hop - offset / hop + 1;
+  if (blocks > 0x7fffffffLL) return cudaErrorInvalidValue;
+  if (x_f64)
+    rms_halfblock_kernel<double><<<(unsigned)blocks, 256, 0, st>>>((const double*)x, len, offset, hop, out);
+  else
+    rms_halfblock_kernel<float><<<(unsigned)blocks, 256, 0, st>>>((const float*)x, len, offset, hop, out);
+  launch_counter().n++;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rms_fold(const double* table, int rows, long long n_hb, int frame_length, float* rms, cudaStream_t st) {
+  if (!table || !rms || rows < 1 || n_hb < 1 || frame_length < 1) return cudaErrorInvalidValue;
+  rms_fold_kernel<<<stream_grid(n_hb, 128), 128, 0, st>>>(table, rows, n_hb, frame_length, rms);
+  launch_counter().n++;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rms_gain(float* x, long long len, long long offset, long long N, const float* rms1, long long n1, const float* rms2,
+                            long long n2, double rate, cudaStream_t st) {
+  if (!x || !rms1 || !rms2 || len < 0 || offset < 0 || N < 1 || offset + len > N || n1 < 1 || n2 < 1 || n1 > 0x7fffffffLL ||
+      n2 > 0x7fffffffLL || !std::isfinite(rate))
+    return cudaErrorInvalidValue;
+  if (len == 0) return cudaSuccess;
+  const float p1 = (float)(1.0 - rate), p2 = (float)(rate - 1.0);
+  rms_gain_kernel<<<stream_grid(len, 256), 256, 0, st>>>(x, len, offset, N, rms1, (int)n1, rms2, (int)n2, p1, p2);
   launch_counter().n++;
   return cudaGetLastError();
 }

@@ -23,6 +23,11 @@ What is different is where the work happens (B200-first, SURVEY.md §8e/§8f-1):
     assigned longest-first to ranks, each rank converts its own, the only cross-segment reduction (`max|x|`, one
     float per rank) and the int16 pieces are gathered on the host; there is no collective on the data path.
   * segmentation is never changed for balance (it would change attention context and break parity).
+  * `rms_mix_rate < 1` (the volume-envelope mix `change_rms`, lib/model_utils.py:39, :183) runs on the device after the
+    segment loop: both envelopes are built from half-second "half-block" sums, so each segment's output contributes its
+    own rows to a [segments][half-blocks] table; under sharding one all-reduce of that table (each element has exactly one
+    non-zero contributor) gives every rank the same envelope bits, and the sharded song stays bit-identical to the
+    unsharded one.  `resample_sr` and `f0_autotune` are not supported.
 
 HuBERT, the f0 estimators and faiss are upstream of this path (SURVEY.md §8f ranks 3-4): `model` is the caller's
 HuBERT object, f0 estimators are looked up in `f0_method_dict` (register callables there) or passed as a
@@ -440,7 +445,7 @@ class VC(FeatureExtractor):
         Under `torch.distributed` every rank must call it with the same arguments; rank 0 (or every rank with
         `all_ranks=True`) returns the song, the others return None."""
         if rms_mix_rate < 1:
-            raise NotImplementedError("rms_mix_rate < 1 (change_rms, lib/model_utils.py:39, needs librosa) is outside this path")
+            self._require_device_mix()
         if resample_sr >= 16000 and tgt_sr != resample_sr:
             raise NotImplementedError("resample_sr (librosa.resample, vc_infer_pipeline.py:185-186) is outside this path")
         dist, rank, world = self._dist()
@@ -471,6 +476,8 @@ class VC(FeatureExtractor):
         self.last_plan = {"opt_ts": list(opt_ts), "segments": segs, "assignment": assignment,
                           "makespan_bound": makespan_bound(lengths, world)}
         staged = self._stage(audio_pad, pitch, pitchf, sid, net_g, staged_audio)               # H2D once per song
+        if rms_mix_rate >= 1:
+            staged.pop("audio64", None)                                                        # only the mix reads it
         t1 = time.time()
         times[1] += t1 - t0                                                                    # :164-165
         ev0 = self._record_event(staged)
@@ -491,11 +498,16 @@ class VC(FeatureExtractor):
             if run:
                 parts.append((s.index, self._convert(staged, model, net_g, s, T_formula, index, big_npy, index_rate,
                                                      version, protect, noise)))
+        sizes = None
+        if world > 1:            # every rank derives all piece sizes from the plan (400 / 320 frame formula of the front end)
+            sizes = [min(s.n_samples // self.window, 2 * hubert_frames(s.n_samples)) * net_g.cfg.upp - 2 * self.t_pad_tgt for s in segs]
+        if rms_mix_rate < 1:                                                                   # :183, before the peak
+            mix_sizes = sizes if sizes is not None else [len(p) for _, p in parts]             # world 1: every part, in order
+            self._rms_mix(staged, parts, mix_sizes, audio.shape[0], tgt_sr, rms_mix_rate, dist, world)
         t_enq = time.time()
         if world > 1 and self._device_collectives(dist, staged):
             # NCCL group: the peak is one 4-byte all-reduce and the int16 pieces travel GPU to GPU (NVLink); rank 0 orders
             # them on the device and does the song's single D2H -- no pickling, no host round trip per rank
-            sizes = [min(s.n_samples // self.window, 2 * hubert_frames(s.n_samples)) * net_g.cfg.upp - 2 * self.t_pad_tgt for s in segs]
             out = self._finalize_gather_device(staged, parts, sizes, assignment, dist, rank, world, all_ranks)
             self._timing(staged, ev0, t0, t_plan, t1, t_enq)
             times[2] += time.time() - t1
@@ -526,6 +538,48 @@ class VC(FeatureExtractor):
         out = np.concatenate([mine_np[i] for i in range(len(segs))])
         times[2] += time.time() - t1
         return out
+
+    # ---- volume-envelope mix (change_rms, lib/model_utils.py:39, vc_infer_pipeline.py:183): host logic ---------------
+    def _rms_mix(self, staged, parts, sizes, n_in: int, tgt_sr: int, rate: float, dist=None, world: int = 1):
+        """Scale this rank's trimmed segment outputs `parts` [(segment index, samples)] in place by
+        rms1 ** (1 - rate) * max(rms2, 1e-6) ** (rate - 1), the reference's `change_rms(audio, 16000, audio_opt, tgt_sr, rate)`.
+
+        librosa.feature.rms with frame_length = 2 * hop (sr // 2 * 2 and sr // 2 for every sr) and centre padding makes frame f
+        the sum of half-blocks f - 1 and f (half-block b = samples [b * hop, (b + 1) * hop)).  rms1 comes from the staged
+        float64 input song (one piece, every rank).  For rms2, segment i (global offset = sum of sizes[:i]) writes its
+        half-block sums into row i of a [segments][half-blocks] float64 table; under sharding the table is all-reduced
+        (each element has one non-zero contributor, so the sum is exact in any order) and the rows are folded in segment
+        order: the same bits on every rank and for every world size.  `sizes`: every segment's output length."""
+        hop1, hop2 = self.sr // 2, int(tgt_sr) // 2
+        offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+        N = int(offs[-1])
+        if N == 0:
+            return
+        for i, p in parts:
+            if len(p) != sizes[i]:
+                raise RuntimeError("HuBERT front end does not follow the 400/320 frame formula; segment sizes cannot be "
+                                   "derived from the plan for the device-side gather")
+        dev = staged["dev"]
+        t1 = torch.zeros(1, 1 + n_in // hop1, dtype=torch.float64, device=dev)
+        x1 = staged["audio64"][self.t_pad: self.t_pad + n_in]                              # the high-passed, unpadded song
+        self._mix_power(staged, x1, 0, hop1, t1[0, : (n_in - 1) // hop1 + 1])
+        rms1 = self._mix_fold(staged, t1, 2 * hop1)
+        t2 = torch.zeros(len(sizes), 1 + N // hop2, dtype=torch.float64, device=dev)
+        for i, p in parts:
+            o, n = int(offs[i]), int(sizes[i])
+            if n:
+                self._mix_power(staged, p, o, hop2, t2[i, o // hop2: (o + n - 1) // hop2 + 1])
+        if world > 1:
+            if self._device_collectives(dist, staged):
+                dist.all_reduce(t2, op=dist.ReduceOp.SUM, group=self.group)
+            else:
+                h = t2.cpu()
+                dist.all_reduce(h, op=dist.ReduceOp.SUM, group=self._gloo_group(dist))
+                if h is not t2:
+                    t2.copy_(h)
+        rms2 = self._mix_fold(staged, t2, 2 * hop2)
+        for i, p in parts:
+            self._mix_gain(staged, p, int(offs[i]), N, rms1, rms2, rate)
 
     # ---- hooks with a host default (the CPU test double overrides the device ones below) ------------------------
     def _plan_song(self, audio: np.ndarray):
@@ -567,6 +621,41 @@ class VC(FeatureExtractor):
         return audio_pad[self.t_pad: self.t_pad + n], audio_pad, opt_ts, segs, audio_d
 
     # ---- device side of the song-level driver (everything below touches the GPU) -----------------------------
+    def _require_device_mix(self):
+        """Checked before planning: the volume-envelope mix has no host implementation."""
+        if torch.device(self.device).type != "cuda":
+            raise NotImplementedError("rms_mix_rate < 1 (change_rms, lib/model_utils.py:39) runs on the device only; "
+                                      "no CPU fallback")
+
+    def _mix_power(self, staged, x, offset: int, hop: int, out):
+        """Half-block sums of float32(x)^2 for the piece x (float32 / float64) at global sample `offset` into `out` (float64,
+        one value per half-block the piece touches), `rvcb200_op_rms_halfblock`."""
+        if x.dtype not in (torch.float32, torch.float64) or not x.is_contiguous() or not out.is_contiguous():
+            raise ValueError("rms mix: contiguous float32 / float64 pieces only")
+        with torch.cuda.device(staged["dev"]):
+            stream = C.c_void_p(torch.cuda.current_stream(staged["dev"]).cuda_stream)
+            _lib.check(_lib.load().rvcb200_op_rms_halfblock(C.c_void_p(x.data_ptr()), 1 if x.dtype == torch.float64 else 0, x.numel(),
+                                                            offset, hop, C.c_void_p(out.data_ptr()), stream), None, "rms_halfblock")
+
+    def _mix_fold(self, staged, table, frame_length: int):
+        """Frame RMS (float32, one per column) of a [rows][half-blocks] table, rows folded in order (`rvcb200_op_rms_fold`)."""
+        rms = torch.empty(table.shape[1], dtype=torch.float32, device=table.device)
+        with torch.cuda.device(staged["dev"]):
+            stream = C.c_void_p(torch.cuda.current_stream(staged["dev"]).cuda_stream)
+            _lib.check(_lib.load().rvcb200_op_rms_fold(C.c_void_p(table.data_ptr()), table.shape[0], table.shape[1], frame_length,
+                                                       C.c_void_p(rms.data_ptr()), stream), None, "rms_fold")
+        return rms
+
+    def _mix_gain(self, staged, x, offset: int, n_total: int, rms1, rms2, rate: float):
+        """x (float32 samples [offset, offset + len) of the n_total-sample song) *= the mix gain, in place (`rvcb200_op_rms_gain`)."""
+        if x.dtype != torch.float32 or not x.is_contiguous():
+            raise ValueError("rms mix: contiguous float32 output pieces only")
+        with torch.cuda.device(staged["dev"]):
+            stream = C.c_void_p(torch.cuda.current_stream(staged["dev"]).cuda_stream)
+            _lib.check(_lib.load().rvcb200_op_rms_gain(C.c_void_p(x.data_ptr()), x.numel(), offset, n_total, C.c_void_p(rms1.data_ptr()),
+                                                       rms1.numel(), C.c_void_p(rms2.data_ptr()), rms2.numel(), float(rate), stream),
+                       None, "rms_gain")
+
     def _record_event(self, staged):
         if staged["dev"].type != "cuda":
             return None
@@ -595,6 +684,7 @@ class VC(FeatureExtractor):
             return {
                 "dev": dev,
                 "audio": audio_d.half() if self.is_half else audio_d.float(),
+                "audio64": audio_d,                                                            # the input envelope of the rms mix
                 "sid": torch.as_tensor(sid).reshape(1).to(dev).long(),                         # :151
                 "pitch": torch.from_numpy(pitch).to(dev).unsqueeze(0) if pitch is not None else None,
                 "pitchf": torch.from_numpy(pitchf).to(dev).unsqueeze(0) if pitchf is not None else None,

@@ -291,6 +291,29 @@ int rvcb200_op_absmax(const float* x, int64_t n, float* out, int32_t reset, void
  * NumPy >= 2 promotion). */
 int rvcb200_op_to_int16(const float* x, int64_t n, const float* absmax, int16_t* out, void* stream);
 
+/* Volume-envelope mix `change_rms` (/root/reference/lib/model_utils.py:39, called at vc_infer_pipeline.py:183):
+ * librosa.feature.rms(frame_length = 2 * hop, hop) is built from half-block sums, half-block b = samples [b * hop, (b + 1) * hop)
+ * of the song, so each segment's output contributes to the envelope on its own.  The three entries below return 1 on a bad
+ * argument. */
+
+/* Half-block power of one piece x[len] of a longer signal, starting at global sample `offset` (x_f64: 0 = float32,
+ * 1 = float64): out[k] = sum of float32(x)^2 over the piece's samples in half-block offset / hop + k, k up to
+ * (offset + len - 1) / hop - offset / hop.  Each square is rounded to float32 (numpy's `np.power(x, 2, dtype=np.float32)`),
+ * the sum is accumulated in double in a fixed order that depends only on the samples' positions within their half-block. */
+int rvcb200_op_rms_halfblock(const void* x, int32_t x_f64, int64_t len, int64_t offset, int32_t hop, double* out, void* stream);
+
+/* Frame RMS from half-block sums split over `rows` rows (table[rows][n_hb], one row per segment): rows added in ascending
+ * order from +0.0, frame f = hb[f - 1] + hb[f] (hb[-1] = 0), rms[f] = sqrt(float32(frame / frame_length)) for f < n_hb,
+ * n_hb = 1 + len / hop (librosa's frame count with center=True). */
+int rvcb200_op_rms_fold(const double* table, int32_t rows, int64_t n_hb, int32_t frame_length, float* rms, void* stream);
+
+/* In place on samples [offset, offset + len) of an N-sample float32 song: x *= pow(e1, 1 - rate) * pow(max(e2, 1e-6), rate - 1),
+ * e1 / e2 = rms1[n1] / rms2[n2] linearly interpolated to N samples with the float32 rounding of torch's CPU
+ * F.interpolate(mode="linear", align_corners=False); exponents float32(1 - rate) / float32(rate - 1); the product and the
+ * update are each one float32 rounding.  powf may differ from torch's CPU pow by an ulp or two. */
+int rvcb200_op_rms_gain(float* x, int64_t len, int64_t offset, int64_t N, const float* rms1, int64_t n1, const float* rms2, int64_t n2,
+                        double rate, void* stream);
+
 /* Measurement aid: while `buf` (device, 16 x grid uint64) is set, every CTA of rvcb200_op_conv_tc launches records globaltimer
  * at 8 fixed points (start, prologue done, producer released, first slab landed, MMAs issued, accumulator complete,
  * epilogue done, exit); NULL switches it off.  tools/trace_generic.py. */
