@@ -132,6 +132,13 @@ SYMBOLS = {
     "rvcb200_op_rms_fold": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]),
     "rvcb200_op_rms_gain": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
                                       C.c_double, C.c_void_p]),
+    "rvcb200_op_ivf_scratch_bytes": (C.c_int64, [C.c_int32, C.c_int32]),
+    "rvcb200_op_ivf_assign": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                        C.c_void_p, C.c_void_p]),
+    "rvcb200_op_ivf_scan": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "rvcb200_op_index_blend": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_void_p, C.c_void_p]),
     "rvcb200_op_hubert_conv0": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                           C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int64, C.c_void_p]),
     "rvcb200_op_layernorm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,

@@ -133,6 +133,17 @@ cudaError_t launch_rms_gain(float* x, long long len, long long offset, long long
 cudaError_t launch_quiet_point(const double* audio_pad, long long lo, long long hi, int window, double* best_v, long long* best_j,
                                int n_blocks, cudaStream_t st);
 
+// ---- index blend of VC.vc, IVF-Flat nprobe 1 (index_kernels.cu) ----
+long long ivf_scratch_bytes(int F, int nlist);
+cudaError_t launch_ivf_assign(const void* x, int x_dtype, long long ldx, int F, int d, const float* cent, const float* cnorm, int nlist,
+                              unsigned long long* coarse, cudaStream_t st);
+cudaError_t launch_ivf_scan(const void* x, int x_dtype, long long ldx, int F, int d, const unsigned long long* coarse, int nlist,
+                            const int* list_offsets, const float* vec, const long long* labels, void* scratch, long long scratch_bytes,
+                            float* score, long long* ix, cudaStream_t st);
+cudaError_t launch_index_blend(const void* feats, int feats_dtype, long long ldf, int F, int d, const float* score, const long long* ix,
+                               const float* vec, const int* pos_of_label, long long ntotal, int is_half, double index_rate, void* out,
+                               cudaStream_t st);
+
 // ---- HuBERT / ContentVec front end, first layer (hubert_kernels.cu) ----
 cudaError_t launch_hubert_conv0(const float* x, const float* w, const float* gn_w, const float* gn_b, double* stats, void* y16,
                                 int B, long long n, int C, int K, int S, float eps, long long y_bstride, cudaStream_t st);

@@ -1205,6 +1205,33 @@ int rvcb200_op_rms_gain(float* x, int64_t len, int64_t offset, int64_t N, const 
   return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
 }
 
+// Index blend (vc_infer_pipeline.py:59-75), IVF-Flat with nprobe 1: fp32 CUDA-core distances, packed-key atomicMin merges.
+int64_t rvcb200_op_ivf_scratch_bytes(int32_t F, int32_t nlist) { return ivf_scratch_bytes(F, nlist); }
+
+int rvcb200_op_ivf_assign(const void* x, int32_t x_dtype, int64_t ldx, int32_t F, int32_t d, const float* centroids, const float* cnorm,
+                          int32_t nlist, uint64_t* coarse, void* stream) {
+  cudaError_t e = launch_ivf_assign(x, x_dtype, ldx, F, d, centroids, cnorm, nlist, reinterpret_cast<unsigned long long*>(coarse),
+                                    reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
+int rvcb200_op_ivf_scan(const void* x, int32_t x_dtype, int64_t ldx, int32_t F, int32_t d, const uint64_t* coarse, int32_t nlist,
+                        const int32_t* list_offsets, const float* vectors, const int64_t* labels, void* scratch, int64_t scratch_bytes,
+                        float* score, int64_t* ix, void* stream) {
+  cudaError_t e = launch_ivf_scan(x, x_dtype, ldx, F, d, reinterpret_cast<const unsigned long long*>(coarse), nlist, list_offsets, vectors,
+                                  reinterpret_cast<const long long*>(labels), scratch, scratch_bytes, score,
+                                  reinterpret_cast<long long*>(ix), reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
+int rvcb200_op_index_blend(const void* feats, int32_t feats_dtype, int64_t ldf, int32_t F, int32_t d, const float* score,
+                           const int64_t* ix, const float* vectors, const int32_t* pos_of_label, int64_t ntotal, int32_t is_half,
+                           double index_rate, void* out, void* stream) {
+  cudaError_t e = launch_index_blend(feats, feats_dtype, ldf, F, d, score, reinterpret_cast<const long long*>(ix), vectors, pos_of_label,
+                                     ntotal, is_half, index_rate, out, reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
 int rvcb200_op_hubert_conv0(const float* x, const float* w, const float* gn_w, const float* gn_b, double* stats, void* y16,
                             int32_t B, int64_t n, int32_t C, int32_t K, int32_t S, float eps, int64_t y_bstride, void* stream) {
   cudaError_t e = launch_hubert_conv0(x, w, gn_w, gn_b, stats, y16, B, n, C, K, S, eps, y_bstride,

@@ -23,6 +23,10 @@ What is different is where the work happens (B200-first, SURVEY.md §8e/§8f-1):
     assigned longest-first to ranks, each rank converts its own, the only cross-segment reduction (`max|x|`, one
     float per rank) and the int16 pieces are gathered on the host; there is no collective on the data path.
   * segmentation is never changed for balance (it would change attention context and break parity).
+  * the index blend (`index_rate > 0`, :59-75) runs on the device when the index is an `IndexIVFFlatB200` (comfy_rvc_b200/index.py:
+    the same IVF-Flat nprobe-1 / flat-L2 top-1 search, gather and blend, enqueued with the segment), passed alone or as the first
+    element of the `(index, big_npy)` tuple; each rank holds its own replica, so sharding needs nothing more.  Any other index
+    (a faiss object, a file path, a test double) keeps the reference's host round trip per segment.
   * `rms_mix_rate < 1` (the volume-envelope mix `change_rms`, lib/model_utils.py:39, :183) runs on the device after the
     segment loop: both envelopes are built from half-second "half-block" sums, so each segment's output contributes its
     own rows to a [segments][half-blocks] table; under sharding one all-reduce of that table (each element has exactly one
@@ -46,6 +50,7 @@ import torch
 from scipy import signal
 
 from . import _lib
+from .index import IndexIVFFlatB200
 
 MAX_INT16 = 32768                                    # lib/audio.py:14
 _BH, _AH = (np.ascontiguousarray(c, dtype=np.float64) for c in signal.butter(N=5, Wn=48, btype="high", fs=16000))   # :21
@@ -222,11 +227,14 @@ class FeatureExtractor:
         return self._rmvpe().infer_from_audio_with_pitch(x, thred=0.03, f0_min=f0_min, f0_max=f0_max)
 
     def load_index(self, file_index):
-        """pitch_extraction.py:49-73: a preloaded `(index, big_npy)` tuple, "" for none, or a faiss file path."""
+        """pitch_extraction.py:49-73: a preloaded `(index, big_npy)` tuple, an `IndexIVFFlatB200` (device blend), "" for none, or a
+        faiss file path."""
         index = big_npy = None
         try:
             if isinstance(file_index, tuple):
                 index, big_npy = file_index
+            elif isinstance(file_index, IndexIVFFlatB200):                                     # the device index alone
+                index = file_index
             elif file_index == "" or file_index is None:
                 index = None
             else:
@@ -339,7 +347,9 @@ class VC(FeatureExtractor):
             noise = noise()      # HuBERT consumes the global generator itself (one torch.rand([]) per encoder layer and forward)
         use_f0 = pitch is not None and pitchf is not None
         feats0 = feats if (protect < 0.5 and use_f0) else None                                 # :57-58 (no clone needed)
-        if index is not None and big_npy is not None and index_rate > 0:                       # :59-75, host like the reference
+        if isinstance(index, IndexIVFFlatB200) and index_rate > 0:                             # :59-75 on the device
+            feats = index.blend(feats, index_rate, self.is_half)
+        elif index is not None and big_npy is not None and index_rate > 0:                     # :59-75, host like the reference
             npy = feats[0].float().cpu().numpy()
             score, ix = index.search(npy, k=1)
             weight = np.square(1 / score)
@@ -815,6 +825,6 @@ def get_vc(model_path, file_index=None, config=None, device=None):
         file_index = vc.load_index(file_index)
         if file_index[0] is None:
             file_index = ""
-    elif not isinstance(file_index, tuple):
+    elif not isinstance(file_index, (tuple, IndexIVFFlatB200)):
         file_index = ""
     return {"vc": vc, "cpt": cpt, "net_g": net_g, "model_name": model_name, "file_index": file_index, "sr": cpt["config"][-1]}

@@ -314,6 +314,39 @@ int rvcb200_op_rms_fold(const double* table, int32_t rows, int64_t n_hb, int32_t
 int rvcb200_op_rms_gain(float* x, int64_t len, int64_t offset, int64_t N, const float* rms1, int64_t n1, const float* rms2, int64_t n2,
                         double rate, void* stream);
 
+/* Index blend of VC.vc (/root/reference/vc_infer_pipeline.py:59-75: `index.search(npy, k=1)`, the `1 / score` weight, the
+ * `big_npy[ix]` gather and the `index_rate` blend) on the device, for a faiss IndexIVFFlat with METRIC_L2 and nprobe 1
+ * (IndexFlatL2 = one list holding every vector in id order).  All distances are fp32 FMA on the CUDA cores; every result is the
+ * same bits for every run.  Queries x: [F] rows of d values (x_dtype / feats_dtype 0 = fp32, 1 = fp16, promoted exactly), row
+ * stride ldx >= d elements; d % 4 == 0.  The index: centroids fp32 [nlist][d], cnorm fp32 [nlist] = ||centroid||^2,
+ * list_offsets int32 [nlist + 1] (CSR, list_offsets[0] = 0), vectors fp32 [ntotal][d] and labels int64 [ntotal] in list order,
+ * pos_of_label int32 [ntotal] = position of label i in `vectors`.  The entries below return 1 on a bad argument and never
+ * allocate: the caller passes the scratch. */
+
+/* Bytes of scratch rvcb200_op_ivf_scan needs for F queries over nlist lists (-1 on a bad argument). */
+int64_t rvcb200_op_ivf_scratch_bytes(int32_t F, int32_t nlist);
+
+/* Coarse step: coarse[f] (uint64 [F]) = key(dist) << 32 | l for the l minimising ||c_l||^2 - 2 x_f . c_l, the lowest l on an
+ * exact tie (key: the order-preserving unsigned image of the fp32 value). */
+int rvcb200_op_ivf_assign(const void* x, int32_t x_dtype, int64_t ldx, int32_t F, int32_t d, const float* centroids, const float* cnorm,
+                          int32_t nlist, uint64_t* coarse, void* stream);
+
+/* Fine step: bucket the queries by the list rvcb200_op_ivf_assign chose, scan each list exhaustively with direct-form
+ * sum_k (x - v)^2, and write score[f] (fp32) = the smallest distance and ix[f] (int64) = its label, the earliest list position
+ * on an exact tie (faiss's heap replaces on a strict <).  A query whose list is empty gets score +inf, ix -1. */
+int rvcb200_op_ivf_scan(const void* x, int32_t x_dtype, int64_t ldx, int32_t F, int32_t d, const uint64_t* coarse, int32_t nlist,
+                        const int32_t* list_offsets, const float* vectors, const int64_t* labels, void* scratch, int64_t scratch_bytes,
+                        float* score, int64_t* ix, void* stream);
+
+/* Blend: out[f][:] (row-contiguous [F][d]) = round(round(g * r) + round(s * feats[f][:])), r = float(index_rate),
+ * s = float(1.0 - index_rate) (the difference taken in double), g = big_npy[ix[f]] * (w / w) with w = float32(1 / score[f])^2
+ * (1.0, or NaN when score is 0, +inf, or w over- / underflows), ix -1 = label ntotal - 1 (numpy's indexing), big_npy[i] =
+ * vectors[pos_of_label[i]].  With is_half, g and g * r are rounded to fp16 (`astype("float16")`); s * f is rounded to the
+ * dtype of feats; out is fp16 when is_half and feats is fp16 (torch's promotion), fp32 otherwise. */
+int rvcb200_op_index_blend(const void* feats, int32_t feats_dtype, int64_t ldf, int32_t F, int32_t d, const float* score,
+                           const int64_t* ix, const float* vectors, const int32_t* pos_of_label, int64_t ntotal, int32_t is_half,
+                           double index_rate, void* out, void* stream);
+
 /* Measurement aid: while `buf` (device, 16 x grid uint64) is set, every CTA of rvcb200_op_conv_tc launches records globaltimer
  * at 8 fixed points (start, prologue done, producer released, first slab landed, MMAs issued, accumulator complete,
  * epilogue done, exit); NULL switches it off.  tools/trace_generic.py. */
