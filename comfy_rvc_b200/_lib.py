@@ -139,6 +139,9 @@ SYMBOLS = {
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rvcb200_op_index_blend": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_void_p, C.c_int64, C.c_int32, C.c_double, C.c_void_p, C.c_void_p]),
+    "rvcb200_op_resample_poly": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_int64,
+                                           C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
+                                           C.c_int64, C.c_void_p, C.c_void_p]),
     "rvcb200_op_hubert_conv0": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                           C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_int64, C.c_void_p]),
     "rvcb200_op_layernorm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,

@@ -130,6 +130,9 @@ cudaError_t launch_rms_halfblock(const void* x, int x_f64, long long len, long l
 cudaError_t launch_rms_fold(const double* table, int rows, long long n_hb, int frame_length, float* rms, cudaStream_t st);
 cudaError_t launch_rms_gain(float* x, long long len, long long offset, long long N, const float* rms1, long long n1, const float* rms2,
                             long long n2, double rate, cudaStream_t st);
+cudaError_t launch_resample_poly(const float* tab, int up, int down, int tpp, long long half_len, const float* left, long long n_left,
+                                 const float* piece, long long n_piece, const float* right, long long n_right, long long piece_off,
+                                 long long n_song, long long out_lo, long long out_hi, float* out, cudaStream_t st);
 cudaError_t launch_quiet_point(const double* audio_pad, long long lo, long long hi, int window, double* best_v, long long* best_j,
                                int n_blocks, cudaStream_t st);
 

@@ -1232,6 +1232,16 @@ int rvcb200_op_index_blend(const void* feats, int32_t feats_dtype, int64_t ldf, 
   return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
 }
 
+// librosa.resample at vc_infer_pipeline.py:185-186, as resample_poly with the filter of comfy_rvc_b200/resample.py: one
+// fixed-order fp32 FMA chain per output, so any split of the output range gives the same bits.
+int rvcb200_op_resample_poly(const float* tab, int32_t up, int32_t down, int32_t tpp, int64_t half_len, const float* left, int64_t n_left,
+                             const float* piece, int64_t n_piece, const float* right, int64_t n_right, int64_t piece_off, int64_t n_song,
+                             int64_t out_lo, int64_t out_hi, float* out, void* stream) {
+  cudaError_t e = launch_resample_poly(tab, up, down, tpp, half_len, left, n_left, piece, n_piece, right, n_right, piece_off, n_song,
+                                       out_lo, out_hi, out, reinterpret_cast<cudaStream_t>(stream));
+  return e == cudaSuccess ? RVCB200_OK : (e == cudaErrorInvalidValue ? RVCB200_ERR_ARG : RVCB200_ERR_CUDA);
+}
+
 int rvcb200_op_hubert_conv0(const float* x, const float* w, const float* gn_w, const float* gn_b, double* stats, void* y16,
                             int32_t B, int64_t n, int32_t C, int32_t K, int32_t S, float eps, int64_t y_bstride, void* stream) {
   cudaError_t e = launch_hubert_conv0(x, w, gn_w, gn_b, stats, y16, B, n, C, K, S, eps, y_bstride,

@@ -3,10 +3,12 @@
 //   absmax        : max |x| over the concatenated song                                 (vc_infer_pipeline.py:188)
 //   to_int16      : x * 32768 / (max / 0.99), C truncation                             (vc_infer_pipeline.py:188-189)
 //   rms_halfblock / rms_fold / rms_gain : the volume-envelope mix `change_rms`      (lib/model_utils.py:39, :183)
-// All of them are HBM-bound streaming kernels (one pass, 16-byte accesses); they exist so that a whole song is
-// converted without a host round trip per segment (the reference syncs and gc's after every segment, :102-112).
+//   resample_poly : polyphase FIR resampling of the song                               (vc_infer_pipeline.py:185-186)
+// All of them but resample_poly (fp32 FMA bound) are HBM-bound streaming kernels (one pass, 16-byte accesses); they exist so
+// that a whole song is converted without a host round trip per segment (the reference syncs and gc's after every segment, :102-112).
 #include <cuda_fp16.h>
 
+#include <algorithm>
 #include <cmath>
 
 #include "common.cuh"
@@ -198,6 +200,81 @@ __global__ void rms_gain_kernel(float* __restrict__ x, long long len, long long 
   }
 }
 
+// ---- output resampling (resample_sr, vc_infer_pipeline.py:185-186) -----------------------------------------------------------
+// y[j] = sum_k tab[r][k] * x[m0 - k], k = 0 .. tpp - 1 in ascending order, one fp32 FMA each, from +0.0, where
+// t = j * down + half_len, r = t % up, m0 = t / up and tab[r][k] = up * h[r + k * up] (comfy_rvc_b200/resample.py).  The sum of
+// an output depends on nothing but j and the input values, so any split of the output range gives the same bits.
+//
+// A CTA owns the outputs [J0, J0 + qb * up).  Outputs j and j + up share a phase and their inputs are `down` apart, so a task
+// is (phase s, 32 consecutive q): lane L computes j = J0 + s + (32 c + L) * up, every lane reads the same tap (a broadcast
+// load) and the inputs x[m0(J0 + s) + (32 c + L) * down - k] from shared memory.  The CTA's input window is staged once, with
+// one padding word after every `down` words when down is even, so that those 32 reads fall in 32 different banks.
+struct ResampleIn {
+  const float* left;
+  const float* piece;
+  const float* right;
+  long long n_left, n_piece, n_right, piece_off, n_song;
+};
+
+__device__ __forceinline__ float resample_fetch(const ResampleIn& in, long long m) {
+  if (m < 0 || m >= in.n_song) return 0.f;
+  const long long rel = m - in.piece_off;
+  if (rel < 0) return rel >= -in.n_left ? in.left[in.n_left + rel] : 0.f;
+  if (rel < in.n_piece) return in.piece[rel];
+  return rel - in.n_piece < in.n_right ? in.right[rel - in.n_piece] : 0.f;
+}
+
+constexpr int kResampleThreads = 256;
+
+__global__ void __launch_bounds__(kResampleThreads) resample_poly_kernel(const float* __restrict__ tab, int up, int down, int tpp,
+                                                                          long long half_len, ResampleIn in, long long out_lo,
+                                                                          long long out_hi, int qb, float* __restrict__ out) {
+  extern __shared__ float xs[];
+  const int stride = (tpp + 3) & ~3;
+  const int pad = (down & 1) ? 0 : 1;
+  const long long J0 = out_lo + (long long)blockIdx.x * qb * up;
+  const long long w_lo = (J0 * down + half_len) / up - (tpp - 1);                  // first input sample of the window
+  const long long w_hi = ((J0 + (long long)up - 1) * down + half_len) / up + (long long)(qb - 1) * down;
+  const int nw = (int)(w_hi - w_lo + 1);
+  for (int i = threadIdx.x; i < nw; i += kResampleThreads) xs[i + pad * (i / down)] = resample_fetch(in, w_lo + i);
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int chunks = qb >> 5;
+  for (int task = warp; task < up * chunks; task += kResampleThreads / 32) {
+    const int s = task % up, c = task / up;
+    const long long js = J0 + s;
+    const long long t = js * down + half_len;
+    const int r = (int)(t % up);
+    const int a = (int)(t / up - w_lo);                                             // local index of m0(js), >= tpp - 1
+    const int q = c * 32 + lane;
+    const float* __restrict__ tr = tab + (long long)r * stride;
+    const float* __restrict__ xl = xs + q * (down + pad);
+    int fu = a + pad * (a / down);                                                  // padded address of local index a - k
+    int col = a % down;
+    float acc = 0.f;
+    int k = 0;
+    for (; k + 4 <= tpp; k += 4) {
+      const float4 w = __ldg(reinterpret_cast<const float4*>(tr + k));
+      const float wk[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        acc = __fmaf_rn(wk[u], xl[fu], acc);
+        fu -= 1;
+        if (col == 0) { fu -= pad; col = down; }
+        col -= 1;
+      }
+    }
+    for (; k < tpp; ++k) {
+      acc = __fmaf_rn(__ldg(tr + k), xl[fu], acc);
+      fu -= 1;
+      if (col == 0) { fu -= pad; col = down; }
+      col -= 1;
+    }
+    const long long j = js + (long long)q * up;
+    if (j < out_hi) out[j - out_lo] = acc;
+  }
+}
+
 inline unsigned stream_grid(long long work, int threads) {
   long long blocks = (work + threads - 1) / threads;
   const long long cap = 148 * 8;
@@ -276,6 +353,39 @@ cudaError_t launch_rms_gain(float* x, long long len, long long offset, long long
   if (len == 0) return cudaSuccess;
   const float p1 = (float)(1.0 - rate), p2 = (float)(rate - 1.0);
   rms_gain_kernel<<<stream_grid(len, 256), 256, 0, st>>>(x, len, offset, N, rms1, (int)n1, rms2, (int)n2, p1, p2);
+  launch_counter().n++;
+  return cudaGetLastError();
+}
+
+cudaError_t launch_resample_poly(const float* tab, int up, int down, int tpp, long long half_len, const float* left, long long n_left,
+                                 const float* piece, long long n_piece, const float* right, long long n_right, long long piece_off,
+                                 long long n_song, long long out_lo, long long out_hi, float* out, cudaStream_t st) {
+  constexpr long long kMaxRate = 1 << 20, kMaxLen = 1LL << 40;
+  if (!tab || (reinterpret_cast<uintptr_t>(tab) & 15) || up < 1 || down < 1 || up > kMaxRate || down > kMaxRate || tpp < 1 ||
+      half_len < 0 || half_len >= (long long)tpp * up || n_left < 0 || n_piece < 0 || n_right < 0 || piece_off < n_left ||
+      n_song > kMaxLen || piece_off + n_piece + n_right > n_song || (n_left && !left) || (n_piece && !piece) ||
+      (n_right && !right) || out_lo < 0 || out_hi < out_lo || out_hi > kMaxLen)
+    return cudaErrorInvalidValue;
+  if (out_hi == out_lo) return cudaSuccess;
+  if (!out) return cudaErrorInvalidValue;
+  // every input sample the outputs [out_lo, out_hi) reach inside the song must be in [left | piece | right]
+  const long long m_first = std::max((out_lo * down + half_len) / up - (tpp - 1), 0LL);
+  const long long m_last = std::min(((out_hi - 1) * down + half_len) / up, n_song - 1);
+  if (m_first <= m_last && (m_first < piece_off - n_left || m_last >= piece_off + n_piece + n_right)) return cudaErrorInvalidValue;
+  // a CTA covers qb * up outputs: about 8 K input words of window, qb a multiple of 32
+  const long long qb = std::max(32LL, (8192LL - tpp) / down / 32 * 32);
+  const long long nw = qb * down + tpp + 1;                                            // window length bound
+  const size_t smem = (size_t)(nw + ((down & 1) ? 0 : nw / down + 1)) * sizeof(float);
+  if (smem > 200 * 1024) return cudaErrorInvalidValue;
+  if (smem > 48 * 1024) {                                                              // per device: set on every such launch
+    cudaError_t e = cudaFuncSetAttribute(resample_poly_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  const long long blocks = (out_hi - out_lo + qb * up - 1) / (qb * up);
+  if (blocks > 0x7fffffffLL) return cudaErrorInvalidValue;
+  const ResampleIn in{left, piece, right, n_left, n_piece, n_right, piece_off, n_song};
+  resample_poly_kernel<<<(unsigned)blocks, kResampleThreads, smem, st>>>(tab, up, down, tpp, half_len, in, out_lo, out_hi, (int)qb,
+                                                                          out);
   launch_counter().n++;
   return cudaGetLastError();
 }

@@ -31,7 +31,15 @@ What is different is where the work happens (B200-first, SURVEY.md §8e/§8f-1):
     segment loop: both envelopes are built from half-second "half-block" sums, so each segment's output contributes its
     own rows to a [segments][half-blocks] table; under sharding one all-reduce of that table (each element has exactly one
     non-zero contributor) gives every rank the same envelope bits, and the sharded song stays bit-identical to the
-    unsharded one.  `resample_sr` and `f0_autotune` are not supported.
+    unsharded one.
+  * `resample_sr` (`librosa.resample`, :185-186, when resample_sr >= 16000 and != tgt_sr) runs on the device after the mix and
+    before the peak: `scipy.signal.resample_poly(x, up, down, window=h)` with the Kaiser-windowed sinc of
+    `comfy_rvc_b200.resample.design` (libsoxr's HQ spec: passband to 0.913 of the lower Nyquist, >= 120 dB stopband from
+    it), one fixed-order fp32 FMA chain per output (`rvcb200_op_resample_poly`).  The reference's soxr_hq resampler cannot
+    be reproduced bit for bit and the distance to it has not been measured.  Segment i owns the outputs
+    [ceil(O_i * up / down), ceil(O_{i+1} * up / down)); the filter's reach into neighbouring segments comes from a
+    [segments][2][halo] table of every piece's first and last samples, all-reduced under sharding like the mix's table, so
+    the sharded song stays bit-identical to the unsharded one.  `f0_autotune` is not supported.
 
 HuBERT, the f0 estimators and faiss are upstream of this path (SURVEY.md §8f ranks 3-4): `model` is the caller's
 HuBERT object, f0 estimators are looked up in `f0_method_dict` (register callables there) or passed as a
@@ -49,7 +57,7 @@ import numpy as np
 import torch
 from scipy import signal
 
-from . import _lib
+from . import _lib, resample
 from .index import IndexIVFFlatB200
 
 MAX_INT16 = 32768                                    # lib/audio.py:14
@@ -306,6 +314,7 @@ class VC(FeatureExtractor):
         self._host_group = None
         self._stage_buf: Optional[torch.Tensor] = None
         self._out_buf: Optional[torch.Tensor] = None
+        self._resample_tables: dict = {}                 # (tgt_sr, resample_sr, device) -> `_resample_table` result
         self.last_plan: Optional[dict] = None
 
     # ---- one segment ------------------------------------------------------------------------------------
@@ -456,8 +465,9 @@ class VC(FeatureExtractor):
         `all_ranks=True`) returns the song, the others return None."""
         if rms_mix_rate < 1:
             self._require_device_mix()
-        if resample_sr >= 16000 and tgt_sr != resample_sr:
-            raise NotImplementedError("resample_sr (librosa.resample, vc_infer_pipeline.py:185-186) is outside this path")
+        resampling = resample_sr >= 16000 and tgt_sr != resample_sr                            # :185
+        if resampling:
+            self._require_device_resample()
         dist, rank, world = self._dist()
         t0 = time.time()
         index, big_npy = self.load_index(file_index)
@@ -514,6 +524,10 @@ class VC(FeatureExtractor):
         if rms_mix_rate < 1:                                                                   # :183, before the peak
             mix_sizes = sizes if sizes is not None else [len(p) for _, p in parts]             # world 1: every part, in order
             self._rms_mix(staged, parts, mix_sizes, audio.shape[0], tgt_sr, rms_mix_rate, dist, world)
+        if resampling:                                                                         # :185-186, before the peak
+            parts, out_sizes = self._resample(staged, parts, sizes if sizes is not None else [len(p) for _, p in parts],
+                                              tgt_sr, resample_sr, dist, world)
+            sizes = out_sizes if sizes is not None else None
         t_enq = time.time()
         if world > 1 and self._device_collectives(dist, staged):
             # NCCL group: the peak is one 4-byte all-reduce and the int16 pieces travel GPU to GPU (NVLink); rank 0 orders
@@ -591,6 +605,65 @@ class VC(FeatureExtractor):
         for i, p in parts:
             self._mix_gain(staged, p, int(offs[i]), N, rms1, rms2, rate)
 
+    # ---- output resampling (librosa.resample, vc_infer_pipeline.py:185-186): host logic ----------------------------------
+    def _resample(self, staged, parts, sizes, tgt_sr: int, resample_sr: int, dist=None, world: int = 1):
+        """Resample this rank's segment outputs `parts` [(segment index, samples)] from tgt_sr to resample_sr
+        (`resample.design`, scipy's resample_poly).  Returns (resampled parts, every segment's resampled size).
+
+        Segment i starts at input sample O_i = sum(sizes[:i]) and owns the outputs [ceil(O_i * up / down),
+        ceil(O_{i+1} * up / down)), an exact partition of the resampled song.  An output's filter reaches up to H samples
+        into the neighbouring segments, which may live on other ranks: each rank writes the first and last H samples of its
+        pieces into their rows of a [segments][2][H] float32 table, zero elsewhere; under sharding the table is all-reduced
+        (one non-zero contributor per element, so the sum is exact) and every segment's halos are assembled from the rows
+        around it.  The same path runs at world size 1, and every output is one fixed-order sum, so the sharded song is
+        bit-identical to the unsharded one.  `sizes`: every segment's input length."""
+        up, down, half_len, tpp, table = self._resample_table(staged, tgt_sr, resample_sr)
+        H = resample.halo_len(2 * half_len + 1, up)
+        offs = np.concatenate([[0], np.cumsum(sizes)]).astype(np.int64)
+        N = int(offs[-1])
+        bounds = [resample.out_len(int(o), up, down) for o in offs]
+        out_sizes = [bounds[i + 1] - bounds[i] for i in range(len(sizes))]
+        for i, p in parts:
+            if len(p) != sizes[i]:
+                raise RuntimeError("HuBERT front end does not follow the 400/320 frame formula; segment sizes cannot be "
+                                   "derived from the plan for the device-side gather")
+        dev = staged["dev"]
+        edges = torch.zeros(len(sizes), 2, H, dtype=torch.float32, device=dev)
+        for i, p in parts:
+            n = min(H, len(p))
+            if n:
+                p_t = torch.as_tensor(p, device=dev)
+                edges[i, 0, :n] = p_t[:n]
+                edges[i, 1, H - n:] = p_t[len(p) - n:]
+        if world > 1:
+            if self._device_collectives(dist, staged):
+                dist.all_reduce(edges, op=dist.ReduceOp.SUM, group=self.group)
+            else:
+                h = edges.cpu()
+                dist.all_reduce(h, op=dist.ReduceOp.SUM, group=self._gloo_group(dist))
+                if h is not edges:
+                    edges.copy_(h)
+        out = []
+        for i, p in parts:
+            left, need, k = [], H, i - 1                                   # the last H samples before segment i
+            while need > 0 and k >= 0:
+                n = min(need, int(sizes[k]))
+                if n:
+                    left.insert(0, edges[k, 1, H - n:])
+                need -= n
+                k -= 1
+            right, need, k = [], H, i + 1                                  # the first H samples after it
+            while need > 0 and k < len(sizes):
+                n = min(need, int(sizes[k]))
+                if n:
+                    right.append(edges[k, 0, :n])
+                need -= n
+                k += 1
+            cat = lambda xs: torch.cat(xs) if xs else edges.new_zeros(0)
+            out.append((i, self._resample_span(staged, table, up, down, tpp, half_len, cat(left), p, cat(right), int(offs[i]), N,
+                                               bounds[i], bounds[i + 1])))
+        return out, out_sizes
+
     # ---- hooks with a host default (the CPU test double overrides the device ones below) ------------------------
     def _plan_song(self, audio: np.ndarray):
         """Planning for `pipeline`: like `plan`, but with a CUDA device the quiet-point search runs there on the staged
@@ -665,6 +738,37 @@ class VC(FeatureExtractor):
             _lib.check(_lib.load().rvcb200_op_rms_gain(C.c_void_p(x.data_ptr()), x.numel(), offset, n_total, C.c_void_p(rms1.data_ptr()),
                                                        rms1.numel(), C.c_void_p(rms2.data_ptr()), rms2.numel(), float(rate), stream),
                        None, "rms_gain")
+
+    def _require_device_resample(self):
+        """Checked before planning: the output resampling has no host implementation."""
+        if torch.device(self.device).type != "cuda":
+            raise NotImplementedError("resample_sr (librosa.resample, vc_infer_pipeline.py:185-186) runs on the device only; "
+                                      "no CPU fallback")
+
+    def _resample_table(self, staged, tgt_sr: int, resample_sr: int):
+        """(up, down, half_len, taps per phase, device phase table) of tgt_sr -> resample_sr, designed once per rate pair and
+        device and kept on this object."""
+        key = (int(tgt_sr), int(resample_sr), staged["dev"])
+        cache = self._resample_tables
+        if key not in cache:
+            up, down, h = resample.design(tgt_sr, resample_sr)
+            tab = torch.from_numpy(resample.phase_table(h, up)).to(staged["dev"])
+            cache[key] = (up, down, (h.shape[0] - 1) // 2, resample.taps_per_phase(h.shape[0], up), tab)
+        return cache[key]
+
+    def _resample_span(self, staged, table, up, down, tpp, half_len, left, piece, right, piece_off: int, n_song: int,
+                       out_lo: int, out_hi: int):
+        """Outputs [out_lo, out_hi) of the resampled song from [left | piece | right] (`rvcb200_op_resample_poly`)."""
+        if any(t.dtype != torch.float32 or not t.is_contiguous() for t in (left, piece, right)):
+            raise ValueError("resample: contiguous float32 pieces only")
+        out = torch.empty(out_hi - out_lo, dtype=torch.float32, device=staged["dev"])
+        ptr = lambda t: C.c_void_p(t.data_ptr() if t.numel() else None)
+        with torch.cuda.device(staged["dev"]):
+            stream = C.c_void_p(torch.cuda.current_stream(staged["dev"]).cuda_stream)
+            _lib.check(_lib.load().rvcb200_op_resample_poly(
+                ptr(table), up, down, tpp, half_len, ptr(left), left.numel(), ptr(piece), piece.numel(), ptr(right), right.numel(),
+                piece_off, n_song, out_lo, out_hi, ptr(out), stream), None, "resample_poly")
+        return out
 
     def _record_event(self, staged):
         if staged["dev"].type != "cuda":

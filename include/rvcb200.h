@@ -347,6 +347,18 @@ int rvcb200_op_index_blend(const void* feats, int32_t feats_dtype, int64_t ldf, 
                            const int64_t* ix, const float* vectors, const int32_t* pos_of_label, int64_t ntotal, int32_t is_half,
                            double index_rate, void* out, void* stream);
 
+/* Output resampling (`resample_sr`, /root/reference/vc_infer_pipeline.py:185-186) as a polyphase FIR:
+ * y[j] = sum_{k < tpp} tab[r][k] * x[m0 - k], t = j * down + half_len, r = t % up, m0 = t / up, k ascending, one fp32 FMA each
+ * from +0.0, so an output's bits depend only on j and the input values (any split of the output range gives the same bits).
+ * tab: device [up][stride] float32, 16-byte aligned, stride = tpp rounded up to 4, row r = up * h[r + k * up]
+ * (comfy_rvc_b200/resample.py `phase_table`).  Computes outputs [out_lo, out_hi) into out[out_hi - out_lo].  The input is the
+ * virtual concatenation [left[n_left] | piece[n_piece] | right[n_right]] whose piece starts at global sample piece_off of an
+ * n_song-sample song; samples outside the song read as zero, and every sample inside the song that the outputs reach must be
+ * in the concatenation.  Returns 1 on a bad argument or an input window that does not cover the outputs. */
+int rvcb200_op_resample_poly(const float* tab, int32_t up, int32_t down, int32_t tpp, int64_t half_len, const float* left, int64_t n_left,
+                             const float* piece, int64_t n_piece, const float* right, int64_t n_right, int64_t piece_off, int64_t n_song,
+                             int64_t out_lo, int64_t out_hi, float* out, void* stream);
+
 /* Measurement aid: while `buf` (device, 16 x grid uint64) is set, every CTA of rvcb200_op_conv_tc launches records globaltimer
  * at 8 fixed points (start, prologue done, producer released, first slab landed, MMAs issued, accumulator complete,
  * epilogue done, exit); NULL switches it off.  tools/trace_generic.py. */
