@@ -268,7 +268,7 @@ class HubertB200:
                                              cur.numel(), self._stream)
             if st != 0:
                 raise RuntimeError(f"rvcb200_op_hubert_conv0 failed with status {st}")
-            self.last_launches += 2
+            self.last_launches += 2 if L <= 256 else 3                        # + the fixed-order reduction of the statistics
             feat32 = None
             nconv = len(self.conv_kernel)
             for i in range(1, nconv):

@@ -371,7 +371,8 @@ int rvcb200_debug_trace_conv_tc(void* buf);
 
 /* First feature-encoder layer: y16[b][t][c] = GELU(GroupNorm_c(sum_k w[c][k] x[b][t*S + k])) as fp16 channels-last,
  * t < L0 = (n - K) / S + 1; per-channel statistics over time, biased variance, affine gn_w / gn_b.  stats: scratch of
- * B * 2 * C doubles; y_bstride: elements between batch items of y16.  K <= 16. */
+ * B * 2 * C doubles; y_bstride: elements between batch items of y16.  K <= 16.  Bitwise deterministic: the statistics are
+ * summed in a fixed order (per-block partial sums are staged in y16 before the outputs overwrite them). */
 int rvcb200_op_hubert_conv0(const float* x, const float* w, const float* gn_w, const float* gn_b, double* stats, void* y16,
                             int32_t B, int64_t n, int32_t C, int32_t K, int32_t S, float eps, int64_t y_bstride, void* stream);
 

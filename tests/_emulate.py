@@ -11,11 +11,11 @@ def conv_cl(x, w, bias=None, g_off=(0,), dil=1, out_stride=1, in_slope=1.0, in_l
     G, ntaps, _, Cout = w.shape
     xa = torch.where(x > 0, x, x * in_slope)
     if in_len is not None:
-        m = (torch.arange(L)[None, :] < in_len[:, None]).to(x.dtype)
+        m = (torch.arange(L, device=x.device)[None, :] < in_len[:, None]).to(x.dtype)
         xa = xa * m[:, :, None]
-    y = torch.zeros(B, L * out_stride, Cout, dtype=x.dtype)
+    y = torch.zeros(B, L * out_stride, Cout, dtype=x.dtype, device=x.device)
     for g in range(G):
-        acc = torch.zeros(B, L, Cout, dtype=x.dtype)
+        acc = torch.zeros(B, L, Cout, dtype=x.dtype, device=x.device)
         for t in range(ntaps):
             off = g_off[g] + t * dil
             lo, hi = max(0, -off), min(L, L - off)

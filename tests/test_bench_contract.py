@@ -51,13 +51,20 @@ def test_reference_arm_dumps_its_last_timed_step(tmp_path):
     w = rvc_oracle.fold_weight_norm(synthetic.make_state_dict(cfg))
     inputs = synthetic.make_inputs(cfg, 1, 20)
     step = lambda seed: rvc_oracle.infer(w, cfg, *inputs, *synthetic.draw_noise(cfg, 1, 20, seed=seed))
-    o, x_mask, (z, z_p, m_p, logs_p) = step(8)
+    # the oracle's CPU reductions depend on the thread count: recompute the step with the reference arm's (bench.py: one
+    # thread per host core), not with whatever this process was started with or an earlier test left behind
+    prev = torch.get_num_threads()
+    torch.set_num_threads(os.cpu_count() or 1)
+    try:
+        o, x_mask, (z, z_p, m_p, logs_p) = step(8)
+        first = step(7)[0].numpy()                   # the first timed step's waveform is a different one
+    finally:
+        torch.set_num_threads(prev)
     want = {"audio": o, "x_mask": x_mask, "z": z, "z_p": z_p, "m_p": m_p, "logs_p": logs_p}
     for name, ref in want.items():
         a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
         assert a.dtype == np.float32 and a.shape == tuple(ref.shape) and np.array_equal(a, b), name
         np.testing.assert_allclose(a, ref.numpy(), rtol=1e-5, atol=1e-5, err_msg=name)
-    first = step(7)[0].numpy()                       # the first timed step's waveform is a different one
     assert np.abs(np.load(tmp_path / "a" / "audio.npy") - first).max() > 1e-3
     out = subprocess.run(args[:4] + ["--steps", "0"], capture_output=True, text=True, env=env, timeout=600, cwd=ROOT)
     assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
