@@ -7,5 +7,6 @@ from .index import IndexIVFFlatB200  # noqa: F401
 from .pipeline import VC, FeatureExtractor, PipelineConfig, get_vc  # noqa: F401
 from .hubert import HubertB200  # noqa: F401
 from .rmvpe import RMVPE  # noqa: F401
+from . import crepe  # noqa: F401
 
-__all__ = ["HubertB200", "IndexIVFFlatB200", "RMVPE", "VC", "FeatureExtractor", "PipelineConfig", "get_vc", "SynthesizerTrnMs256NSFsid", "SynthesizerTrnMs768NSFsid", "SynthesizerTrnMs256NSFsid_nono", "SynthesizerTrnMs768NSFsid_nono", "SynthesizerB200", "SynthConfig", "NAMED_CONFIGS"]
+__all__ = ["crepe", "HubertB200", "IndexIVFFlatB200", "RMVPE", "VC", "FeatureExtractor", "PipelineConfig", "get_vc", "SynthesizerTrnMs256NSFsid", "SynthesizerTrnMs768NSFsid", "SynthesizerTrnMs256NSFsid_nono", "SynthesizerTrnMs768NSFsid_nono", "SynthesizerB200", "SynthConfig", "NAMED_CONFIGS"]

@@ -113,6 +113,12 @@ SYMBOLS = {
                                           C.c_void_p]),
     "rvcb200_op_rmvpe_mel_to_img": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_int32, C.c_int32,
                                               C.c_void_p]),
+    "rvcb200_op_crepe_frames": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "rvcb200_op_crepe_bn_pool": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32,
+                                           C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
+    "rvcb200_op_crepe_decode": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "rvcb200_op_rbconv_tc": (C.c_int, [C.POINTER(TcConvDesc), C.c_int32, C.c_void_p]),
     "rvcb200_op_rbpair_tc": (C.c_int, [C.POINTER(TcConvDesc), C.POINTER(TcConvDesc), C.c_int32, C.c_void_p]),
     "rvcb200_op_sine_scratch_bytes": (C.c_int64, [C.c_int32, C.c_int32, C.c_int32]),

@@ -166,4 +166,14 @@ cudaError_t launch_rmvpe_decode(const float* in, int ld, int from_hidden, float*
 cudaError_t launch_rmvpe_mel_to_img(const float* mel, void* img, int n_frames, int frames_out, float bn_scale, float bn_shift,
                                     int img_pitch, int img_c, cudaStream_t st);
 
+// ---- CREPE f0 estimator: the non-contraction steps (crepe_kernels.cu) ----
+cudaError_t launch_crepe_frames(const float* audio, long long n, long long first, long long count, int hop, int pad, void* out,
+                                cudaStream_t st);
+cudaError_t launch_crepe_bn_pool(const void* x, const float* scale, const float* shift, void* out, long long frames, int C, int L,
+                                 int p_in, int in_off, int p_out, int out_off, cudaStream_t st);
+cudaError_t launch_crepe_decode(const float* in, int ld, int from_salience, long long T, int chunk, int lo, int hi, int mode,
+                                const double* dither, const double* wcents, const double* ltab, double c_out, double log_init,
+                                float* sal, double* logp, unsigned short* ptr, int* bins, double* f0, float* period, double* score,
+                                cudaStream_t st);
+
 }  // namespace rvc

@@ -1300,6 +1300,28 @@ int rvcb200_op_rmvpe_decode(const float* in, int32_t ld, int32_t from_hidden, fl
   RVC_RET(e);
 }
 
+int rvcb200_op_crepe_frames(const float* audio, int64_t n, int64_t first, int64_t count, int32_t hop, int32_t pad, void* frames16,
+                            void* stream) {
+  cudaError_t e = launch_crepe_frames(audio, n, first, count, hop, pad, frames16, reinterpret_cast<cudaStream_t>(stream));
+  RVC_RET(e);
+}
+
+int rvcb200_op_crepe_bn_pool(const void* x16, const float* scale, const float* shift, void* y16, int64_t frames, int32_t C, int32_t L,
+                             int32_t p_in, int32_t in_off, int32_t p_out, int32_t out_off, void* stream) {
+  cudaError_t e = launch_crepe_bn_pool(x16, scale, shift, y16, frames, C, L, p_in, in_off, p_out, out_off,
+                                       reinterpret_cast<cudaStream_t>(stream));
+  RVC_RET(e);
+}
+
+int rvcb200_op_crepe_decode(const float* in, int32_t ld, int32_t from_salience, int64_t T, int32_t chunk, int32_t lo, int32_t hi,
+                            int32_t mode, const double* dither, const double* wcents, const double* log_trans, double log_out,
+                            double log_init, float* salience, double* logp, uint16_t* ptr, int32_t* bins, double* f0, float* periodicity,
+                            double* score, void* stream) {
+  cudaError_t e = launch_crepe_decode(in, ld, from_salience, T, chunk, lo, hi, mode, dither, wcents, log_trans, log_out, log_init,
+                                      salience, logp, ptr, bins, f0, periodicity, score, reinterpret_cast<cudaStream_t>(stream));
+  RVC_RET(e);
+}
+
 int rvcb200_op_rmvpe_mel_to_img(const float* mel, void* img16, int32_t n_frames, int32_t frames_out, float bn_scale, float bn_shift,
                                 int32_t img_pitch, int32_t img_c, void* stream) {
   cudaError_t e = launch_rmvpe_mel_to_img(mel, img16, n_frames, frames_out, bn_scale, bn_shift, img_pitch, img_c,

@@ -75,6 +75,7 @@ class PipelineConfig:
     is_half: bool = True
     device: str = "cuda:0"
     rmvpe_model_path: Optional[str] = None     # BASE_MODELS_DIR/rmvpe.pt in the reference (pitch_extraction.py:193)
+    crepe_model_path: Optional[str] = None     # torchcrepe's assets/full.pth (f0_method "crepe")
 
     @classmethod
     def for_device(cls, is_half: bool = True, gpu_mem_gb: Optional[int] = None, device: str = "cuda:0") -> "PipelineConfig":
@@ -213,9 +214,11 @@ class FeatureExtractor:
         self.onnx = onnx
         # the reference registers pm/harvest/dio/rmvpe/crepe here (pitch_extraction.py:28-45).  RMVPE -- the nodes' default
         # (custom_nodes/rvc_nodes.py:49) -- runs on the B200 kernels (comfy_rvc_b200/rmvpe.py); the CPU estimators (parselmouth,
-        # pyworld, torchcrepe) are upstream of this path: register any callable `fn(x=, f0_up_key=, f0_min=, f0_max=, ...) -> f0[frames]`
-        self.f0_method_dict = {"rmvpe": self.get_rmvpe, "rmvpe+": self.get_pitch_dependant_rmvpe}
+        # pyworld) are upstream of this path: register any callable `fn(x=, f0_up_key=, f0_min=, f0_max=, ...) -> f0[frames]`.
+        # CREPE runs on the B200 kernels too (comfy_rvc_b200/crepe.py).
+        self.f0_method_dict = {"rmvpe": self.get_rmvpe, "rmvpe+": self.get_pitch_dependant_rmvpe, "crepe": self.get_crepe}
         self.rmvpe_model_path = getattr(config, "rmvpe_model_path", None)
+        self.crepe_model_path = getattr(config, "crepe_model_path", None)
 
     def _rmvpe(self):
         """pitch_extraction.py:192-193: built on first use and kept; attach a ready model as `self.model_rmvpe` to share it."""
@@ -233,6 +236,34 @@ class FeatureExtractor:
     def get_pitch_dependant_rmvpe(self, x, f0_min=0, f0_max=40000, *args, **kwargs):
         """pitch_extraction.py:197-201."""
         return self._rmvpe().infer_from_audio_with_pitch(x, thred=0.03, f0_min=f0_min, f0_max=f0_max)
+
+    def _crepe(self):
+        """Built on first use and kept, like `_rmvpe`; attach a ready `comfy_rvc_b200.crepe.Crepe("full")` as `self.model_crepe`
+        to share it.  Without either, the weights registered with `crepe.load_weights("full", ...)` (or an installed
+        torchcrepe's) are used."""
+        if not hasattr(self, "model_crepe"):
+            from . import crepe
+            self.model_crepe = crepe.Crepe("full", weights=self.crepe_model_path, device=self.device)
+        return self.model_crepe
+
+    def get_crepe(self, x, f0_min=50, f0_max=1100, crepe_hop_length=160, model="full", **kwargs):
+        """f0 by CREPE on the device.  The assumed recipe (the RVC-lineage `get_f0_crepe_computation`; the reference's own
+        wrapper was not available when this was written) -- change it here and nowhere else:
+          1. x = float32(x) / quantile(|x|, 0.999);
+          2. predict(x, 16000, crepe_hop_length, f0_min, f0_max, "full", batch_size = 2 * crepe_hop_length, pad=True)
+             (Viterbi decode);
+          3. values < 0.001 -> NaN;  4. np.interp onto p_len = len(x) // 160 frames;  5. nan_to_num."""
+        from . import crepe
+        x = x.astype(np.float32)
+        x /= np.quantile(np.abs(x), 0.999)
+        audio = torch.from_numpy(x)[None]
+        pitch = crepe.predict(audio, self.sr, crepe_hop_length, f0_min, f0_max, model, batch_size=crepe_hop_length * 2,
+                              device=self.device, pad=True, crepe_model=self._crepe())
+        source = np.array(pitch.squeeze(0).cpu().float().numpy())
+        source[source < 0.001] = np.nan
+        p_len = x.shape[0] // self.window
+        target = np.interp(np.arange(0, len(source) * p_len, len(source)) / p_len, np.arange(0, len(source)), source)
+        return np.nan_to_num(target)
 
     def load_index(self, file_index):
         """pitch_extraction.py:49-73: a preloaded `(index, big_npy)` tuple, an `IndexIVFFlatB200` (device blend), "" for none, or a

@@ -396,3 +396,51 @@ def make_rmvpe_state_dict(seed: int = 0, **arch) -> Dict[str, torch.Tensor]:
         else:
             sd[k] = rn(*shape) * math.sqrt(2.0 / _fan_in(shape))
     return sd
+
+
+# ---- CREPE (torchcrepe's `full` / `tiny`) ------------------------------------------------------------------------------------
+def crepe_state_dict_shapes(model: str = "full") -> Dict[str, Tuple[int, ...]]:
+    """Key -> shape of torchcrepe's `Crepe(model)` state dict, in module order."""
+    cin, cout, nf = {"full": ([1, 1024, 128, 128, 128, 256], [1024, 128, 128, 128, 256, 512], 2048),
+                     "tiny": ([1, 128, 16, 16, 16, 32], [128, 16, 16, 16, 32, 64], 256)}[model]
+    s: Dict[str, Tuple[int, ...]] = {}
+    for i in range(6):
+        s[f"conv{i + 1}.weight"] = (cout[i], cin[i], 512 if i == 0 else 64, 1)
+        s[f"conv{i + 1}.bias"] = (cout[i],)
+        for k in ("weight", "bias", "running_mean", "running_var"):
+            s[f"conv{i + 1}_BN.{k}"] = (cout[i],)
+        s[f"conv{i + 1}_BN.num_batches_tracked"] = ()
+    s["classifier.weight"], s["classifier.bias"] = (360, nf), (360,)
+    return s
+
+
+def make_crepe_state_dict(seed: int = 0, model: str = "full") -> Dict[str, torch.Tensor]:
+    """Seeded CREPE weights in torchcrepe's layout (the real `full.pth` is not available offline).  He-scaled convolutions,
+    BatchNorm statistics near what a ReLU output of that scale has (so every layer's output stays O(1)), BatchNorm gains of
+    both signs on a few channels (exercising the sign of the scale), and a classifier scaled so that the logits spread over
+    several units: the median gap between the two largest in-range logits is far above the fp16 path's error."""
+    g = torch.Generator().manual_seed(2000 + seed)
+    rn = lambda *shape: torch.randn(*shape, generator=g)
+    ru = lambda *shape: torch.rand(*shape, generator=g)
+    sd: Dict[str, torch.Tensor] = {}
+    for k, shape in crepe_state_dict_shapes(model).items():
+        if k.endswith("num_batches_tracked"):
+            sd[k] = torch.tensor(0, dtype=torch.long)
+        elif k.endswith("running_mean"):
+            sd[k] = 0.4 + 0.1 * rn(*shape)
+        elif k.endswith("running_var"):
+            sd[k] = 0.3 + 0.2 * ru(*shape)
+        elif "_BN.weight" in k:
+            w = 0.8 + 0.4 * ru(*shape)
+            sd[k] = torch.where(ru(*shape) < 0.05, -w, w)
+        elif "_BN.bias" in k:
+            sd[k] = 0.1 * rn(*shape)
+        elif k == "classifier.weight":
+            sd[k] = rn(*shape) * 1.5 / math.sqrt(shape[1])
+        elif k == "classifier.bias":
+            sd[k] = -1.0 + 0.5 * rn(*shape)
+        elif k.endswith("bias"):
+            sd[k] = 0.05 * rn(*shape)
+        else:
+            sd[k] = rn(*shape) * math.sqrt(2.0 / _fan_in(shape))
+    return sd

@@ -430,6 +430,33 @@ int rvcb200_op_rmvpe_decode(const float* in, int32_t ld, int32_t from_hidden, fl
 int rvcb200_op_rmvpe_mel_to_img(const float* mel, void* img16, int32_t n_frames, int32_t frames_out, float bn_scale, float bn_shift,
                                 int32_t img_pitch, int32_t img_c, void* stream);
 
+/* ---- CREPE f0 estimator (torchcrepe's model, framing and decoders; host orchestration in comfy_rvc_b200/crepe.py) ----
+ * conv1..conv6 and the classifier run through rvcb200_op_conv_tc; these entries are what is left. */
+
+/* Frames first .. first + count - 1 of 16 kHz audio[n] at `hop` (pad != 0: the audio is zero-padded by 512 on each side),
+ * each mean-subtracted and divided by max(1e-10, unbiased std), written as conv1's operand: fp16 [count][368][64] with
+ * row t, channel c = frame[4 t + c - 254] (0 outside the frame).  conv1 is then 8 taps at dilation 16 over these rows. */
+int rvcb200_op_crepe_frames(const float* audio, int64_t n, int64_t first, int64_t count, int32_t hop, int32_t pad, void* frames16,
+                            void* stream);
+
+/* Eval-mode BatchNorm (y = x * scale + shift per channel) then max_pool (2, 1): x16 fp16 rows [frames * p_in][C], frame f's
+ * L rows from row f * p_in + in_off -> y16 fp16 [frames][p_out][C], rows out_off .. out_off + L / 2 - 1 hold the pooled
+ * values, every other row is written as 0 (the zero padding of the next convolution).  C % 8 == 0, L even. */
+int rvcb200_op_crepe_bn_pool(const void* x16, const float* scale, const float* shift, void* y16, int64_t frames, int32_t C, int32_t L,
+                             int32_t p_in, int32_t in_off, int32_t p_out, int32_t out_off, void* stream);
+
+/* torchcrepe's postprocess for T frames: salience s = sigmoid(in) (from_salience != 0: in already is s) [T][ld >= 360], bins
+ * outside [lo, hi) masked; mode 0 = argmax, 1 = weighted_argmax (wcents[360]: the dithered cents of each bin), 2 = Viterbi
+ * over chunks of `chunk` frames (log_trans [360][23]: log(transition + tiny) of bin k to bin k + d - 11, log_out: the same outside
+ * the band, log_init: log(1 / 360 + tiny); the observations log(softmax + tiny) in float64).  Outputs: bins int32 [T],
+ * f0 float64 [T] (Hz; modes 0 / 2: from 20 bin + 1997.379... + dither[t] cents), periodicity fp32 [T] (the salience at the
+ * bin, may be NULL).  salience fp32 [T][360] may be NULL except in mode 2; mode 2 also needs logp float64 [T][360],
+ * ptr uint16 [T][360] and score float64 [chunks] (the log-probability of each chunk's best path). */
+int rvcb200_op_crepe_decode(const float* in, int32_t ld, int32_t from_salience, int64_t T, int32_t chunk, int32_t lo, int32_t hi,
+                            int32_t mode, const double* dither, const double* wcents, const double* log_trans, double log_out,
+                            double log_init, float* salience, double* logp, uint16_t* ptr, int32_t* bins, double* f0, float* periodicity,
+                            double* score, void* stream);
+
 /* ---- host (CPU) side of the song-level driver (csrc/host_plan.cu) ---- */
 
 /* Quiet-point search of /root/reference/vc_infer_pipeline.py:127-135: the first j in [lo, hi) (returned relative to lo)
